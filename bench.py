@@ -19,6 +19,11 @@ load the product library; their thread count is set explicitly (torchrun exports
 With N > 1 the frame is partitioned into interleaved tiles (strong scaling); the timed region includes the exchange: every
 rank stores its pixels straight into rank 0's frame over NVLink peer memory and signals arrival with a flag
 (CGRT_EXCHANGE=nccl selects the NCCL gather + de-interleave kernel instead).
+
+The benchmark runs what __graft_entry__.build() left in the tree and writes nothing into an up-to-date tree (it may be
+read-only); a build older than its sources is redone first where the tree can be written.
+`--dump-outputs DIR` writes what the last timed frame delivered (DIR/frame.npy, DIR/ray_counts.npy): the inputs are fixed,
+so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -33,6 +38,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # no __pycache__ next to the sources
 
 import __graft_entry__ as ge  # noqa: E402
 
@@ -133,10 +139,24 @@ def cpu_threads():
         return max(1, os.cpu_count() or 1)
 
 
+def use_build(product=True):
+    """Run what build() left: nothing is written into a tree that is up to date. A build older than its sources is redone
+    (build_checkers() alone for the CPU legs, which never load the product library) when the tree can be written;
+    a read-only tree is used as it is, with a warning."""
+    if not ge.stale(product):
+        return
+    if not os.access(ROOT, os.W_OK):
+        sys.stderr.write("bench.py: the built libraries are older than their sources and the tree is read-only: using them as built\n")
+    elif product:
+        ge.build()  # every rank: serialised by a file lock
+    else:
+        ge.build_checkers()
+
+
 def cpu_checker():
     """oracle/_ref (the reference's own compiled TUs) when present, else the restatement. Test infrastructure: this is the
     only place besides tests/ and smoke() where bench.py touches oracle/. Never loads the product library."""
-    ge.build_checkers()
+    use_build(product=False)
     from oracle import bindings as ob
     try:
         return ob.RefLib(), "reference", ob
@@ -189,9 +209,20 @@ def frame_parity(rgb, counters, ref_rgb, ref_cnt):
             "tolerance": "max_abs <= 1/255, bit_equal_frac >= 0.999 (pow() in the specular term is the only inexact op)"}
 
 
+def write_outputs(path, arrays):
+    """DIR/<name>.npy for each array of the last timed step: `frame` = the float32 [HEIGHT, WIDTH, 3] frame the timed call
+    leaves on rank 0 (24.9 MB), `ray_counts` = primary, primary_hit, shadow, bounce rays of that frame over all ranks (float64)."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
+
+
 def run_reference(args):
     lib, kind, ob, flat, lights, b = cpu_scene()
-    v, nt, rays, dt, n, _, _ = cpu_frames(b, ob, args.steps, args.warmup)
+    v, nt, rays, dt, n, rgb, cnt = cpu_frames(b, ob, args.steps, args.warmup)
+    if args.dump_outputs:
+        counts = np.array([cnt[k] for k in ("primary", "primary_hit", "shadow", "bounce")], np.float64)
+        write_outputs(args.dump_outputs, {"frame": rgb, "ray_counts": counts})
     line = {
         "impl": "reference", "metric": METRIC, "value": v, "unit": "Mrays/s", "n_gpus": args.gpus, "steps": args.steps,
         "warmup": args.warmup, "ms_per_step": dt / max(n, 1) * 1e3, "higher_is_better": True, "scaling": "strong",
@@ -211,7 +242,10 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed frame's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -221,7 +255,7 @@ def main():
         if rank == 0:  # the CPU arm runs on rank 0 alone; the other ranks exit without work. The product library is not loaded.
             run_reference(args)
         return
-    ge.build()  # every rank: serialised by a file lock, a no-op time-stamp check when the built files shipped with the snapshot
+    use_build()
 
     import torch
     import torch.distributed as dist
@@ -295,13 +329,18 @@ def main():
     for k in range(args.steps):
         flush.zero_()
         ev[k][0].record()
-        R.render_device(cam, flags=(1 << dominant))
+        frame = R.render_device(cam, flags=(1 << dominant))
         ev[k][1].record()
         st = scene.collect_stats()  # synchronises the frame; reads the dominant kernel's event times
         dom_ms += st["class_ms"][dominant]
         dom_launches += st["class_launches"][dominant]
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:  # copied now: the frame buffers are reused by the frames below
+        counts = torch.tensor([st[k] for k in ("primary", "primary_hit", "shadow", "bounce")], dtype=torch.float64, device=dev)
+        if world > 1:
+            dist.all_reduce(counts, op=dist.ReduceOp.SUM)
+        dump = {"frame": frame.cpu().numpy().reshape(HEIGHT, WIDTH, 3), "ray_counts": counts.cpu().numpy()} if rank == 0 else None
     total_ms = sum(a.elapsed_time(b) for a, b in ev)
     t = torch.tensor([total_ms], dtype=torch.float64, device=dev)
     if world > 1:
@@ -441,6 +480,8 @@ def main():
                                     "sample_rays": rays, "sample_seconds": secs}
             line["parity"] = frame_parity(gpu_frame, {"primary": n_primary, "shadow": n_shadow, "bounce": n_bounce}, ref_rgb, ref_cnt)
             line["parity"]["cpu_scene_equals_gpu_scene"] = fixture_ok
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, dump)
         print(json.dumps(line))
     if world > 1:
         dist.barrier(device_ids=[local_rank])

@@ -14,7 +14,8 @@ import __graft_entry__ as ge  # noqa: E402
 from oracle import bindings as ob  # noqa: E402
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-REFERENCE_DATA = "/root/reference/data"
+# data/ of a CG-RayTracer checkout (its OBJ/MTL files are not part of this repository); the loader tests skip without it
+REFERENCE_DATA = os.environ.get("CGRT_REFERENCE_DATA", "")
 
 
 def pytest_configure(config):
@@ -38,11 +39,11 @@ def oracle():
 
 @pytest.fixture(scope="session")
 def reflib():
-    """The reference's own TUs compiled verbatim; present wherever oracle/_ref was built (here) or shipped (GPU box)."""
+    """The reference's own TUs compiled verbatim (oracle/_ref, built where the reference's sources are present), else None."""
     try:
         return ob.RefLib()
     except (FileNotFoundError, OSError):
-        pytest.skip("oracle/_ref/libcgrt_ref.so not available")
+        return None
 
 
 @pytest.fixture(scope="session")

@@ -11,7 +11,10 @@ For every bundled scene the fixture stores
   * outputs of the verbatim reference code on it: BVH node table (reference CONSTRUCTOR, mode 0), leaf triangle orders,
     closest-hit records + per-ray box/triangle test counts for a ray set (primary rays of a small frame + random rays),
     rendered frames at trace limits 1, 2 and 5 with ray counters,
-and one file of unit-function vectors (random + adversarial) with the verbatim functions' answers.
+and one file of unit-function vectors (random + adversarial) with the verbatim functions' answers, and vs_reference.npz:
+the outputs tests/test_oracle_vs_reference.py compares on its seeded soups and on the empty scene with spheres
+(`--vs-reference-from-restatement` writes that file from oracle/liboracle.so where the reference is not available;
+its `source` entry says which).
 """
 import os
 import sys
@@ -116,9 +119,62 @@ def scene_fixture(R, capi, name, hs, frame, nrand, rng, lights=None, use_ctor=Tr
     return out
 
 
+VS_REFERENCE_CASES = [(1, 1, 0.5, 4), (2, 1, 0.5, 5), (3, 1, 0.4, 6), (7, 3, 0.5, 7), (500, 1, 0.1, 8), (900, 40, 0.2, 9),
+                      (2500, 2, 0.05, 10)]  # (triangles, meshes, scale, seed) of tests/test_oracle_vs_reference.py
+VS_REFERENCE_LIGHTS = np.array([[0.0, 0.9, 0.0, 1, 1, 1], [-1, 1, -1, 0.5, 0.5, 0.5]], np.float32)
+SPHERES_PRESET = [[3, -2, 10.2, 1, .8, .2, .2, 0, 0, 0, 1, 1], [-2, 2, 4, 2, .6, .8, .2, 0, 0, 0, 1, 1],
+                  [0, 0, 6, .75, .2, .2, .8, 0, 0, 0, 1, 1]]  # src/scene.cpp:51-56
+
+
+def vs_reference_inputs(ntri, nmesh, scale, seed):
+    """scene and rays of one case of test_tree_hits_images (generated from seeds, not stored)"""
+    flat = ob.random_soup(ntri, seed=seed, scale=scale, n_meshes=nmesh)
+    rays = ob.random_rays(5000, seed=seed + 100)
+    rays["t"][::7] = np.float32(0.7)
+    return flat, rays
+
+
+def empty_scene_inputs():
+    """the Spheres preset without meshes and the rays of test_empty_scene_and_spheres"""
+    empty = ob.FlatScene(np.zeros(0, np.int32), np.zeros(0, np.int32), np.zeros((0, 6)), np.zeros((0, 3)), np.zeros((0, 8)),
+                         spheres=SPHERES_PRESET)
+    rays = ob.random_rays(4000, seed=1)
+    rays["o"][:, 2] -= 3
+    return empty, rays
+
+
+def vs_reference_vectors(R):
+    """What tests/test_oracle_vs_reference.py compares: for every seeded soup the tree of the reference CONSTRUCTOR (mode 0),
+    its leaf orders, closest hits + per-ray test counts of 5000 rays, the 64x48 frame at trace limit 3 and its ray counters;
+    for the empty scene with the Spheres preset, t and n of 4000 rays."""
+    out = {}
+    for ntri, nmesh, scale, seed in VS_REFERENCE_CASES:
+        flat, rays = vs_reference_inputs(ntri, nmesh, scale, seed)
+        b = R.scene(flat, VS_REFERENCE_LIGHTS).bvh(mode=0)
+        meta, aabb = b.nodes()
+        leaves = np.nonzero(meta[:, 0])[0]
+        hits, counts = b.intersect(rays, counts=True)
+        img, cnt = b.render(ob.default_camera(64, 48), 64, 48, trace_limit=3, duplicate_shading=True)
+        k = f"s{seed}_"
+        out.update({k + "node_meta": meta, k + "node_aabb": aabb,
+                    k + "leaf_tris": np.concatenate([b.leaf_triangles(i, meta[i, 4]) for i in leaves]),
+                    k + "hits": hits, k + "counts": counts, k + "img_L3": img,
+                    k + "cnt_L3": np.array([cnt[c] for c in ("primary", "primary_hit", "shadow", "bounce")], np.uint64)})
+    empty, rays = empty_scene_inputs()
+    h = R.scene(empty).bvh(mode=0).intersect(rays)
+    out.update(empty_t=h["t"], empty_n=h["n"])
+    return out
+
+
+def write_vs_reference(R, source):
+    np.savez_compressed(os.path.join(HERE, "vs_reference.npz"), source=np.array(source), **vs_reference_vectors(R))
+    print(f"vs_reference.npz written ({source}), {os.path.getsize(os.path.join(HERE, 'vs_reference.npz')) / 1e6:.2f} MB")
+
+
 def main():
     capi = ge.load_package().capi
     R = ob.RefLib()
+    write_vs_reference(R, "reference")
     rng = np.random.default_rng(20261018)
     np.savez_compressed(os.path.join(HERE, "units.npz"), **unit_vectors(R, rng))
     print("units.npz written")
@@ -147,4 +203,9 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:] == ["--vs-reference-from-restatement"]:
+        # without the reference's sources: the restatement's outputs, which test_oracle_vs_reference checked bit-equal to
+        # the reference's own on exactly these inputs while oracle/_ref was built
+        write_vs_reference(ob.OracleLib(), "restatement, bit-identical to the reference on these inputs")
+    else:
+        main()

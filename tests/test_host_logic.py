@@ -133,7 +133,7 @@ def test_tile_partition_rejects_bad_arguments(capi):
     assert capi.tile_buffer_floats(capi.render_params(0, 64, 2, 0, 1)) == 0
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE_DATA), reason="reference checkout not present (GPU box)")
+@pytest.mark.skipif(not os.path.isdir(REFERENCE_DATA), reason="CGRT_REFERENCE_DATA does not name a CG-RayTracer data/ directory")
 @pytest.mark.parametrize("name,preset", [("triangle", "SingleTriangle"), ("cube", "Cube"), ("cornell", "CornellBox"),
                                          ("monkey", "Monkey")])
 def test_loader_reproduces_fixture_scenes(capi, name, preset):
@@ -144,7 +144,7 @@ def test_loader_reproduces_fixture_scenes(capi, name, preset):
     assert same_bits(hs.materials, g.flat.materials) and same_bits(hs.lights, g.lights)
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE_DATA), reason="reference checkout not present (GPU box)")
+@pytest.mark.skipif(not os.path.isdir(REFERENCE_DATA), reason="CGRT_REFERENCE_DATA does not name a CG-RayTracer data/ directory")
 def test_loader_details(capi):
     c = capi.load_preset("CornellBox", REFERENCE_DATA)
     # unit normalisation (mesh.cpp:143-166): farthest vertex at distance 1 from the mean of all (duplicated) vertices
