@@ -191,10 +191,12 @@ def make_camera(W, H, fovy_deg=50.0, dist=3.0, look_at=(0.0, 0.0, 0.0), euler_de
 
 
 K_PRIMARY, K_BOUNCE, K_SHADOW, K_SHADE = 0, 1, 2, 3
-# production (path pipeline) kernels per class; class 1 is only launched by the level-by-level counting pipeline
-KERNEL_CLASS_NAMES = ["k_paths", "k_bounce_closest", "k_shadow_all", "k_shade_paths"]  # path pipeline (exact-only scenes)
-ROUND_CLASS_NAMES = ["k_gen", "k_finish", "k_trace", "k_shade_slots"]                   # round pipeline (CGRT_PIPELINE=rounds)
-WAVE_CLASS_NAMES = ["-", "-", "k_wave", "-"]                                             # persistent wavefront (production)
+# kernels per class of each pipeline, indexed by cgrt_render_stats.pipeline (0 count, 1 paths, 2 rounds, 3 k_wave). Frames of
+# scenes with a search tree run k_wave or the round pipeline, chosen per frame (DESIGN 4.4); the path pipeline launches no
+# class-1 kernel (k_paths follows each path through its bounces)
+KERNEL_CLASS_NAMES = ["k_paths", "k_bounce_closest", "k_shadow_all", "k_shade_paths"]  # path pipeline (scenes without a search tree)
+ROUND_CLASS_NAMES = ["k_gen", "k_finish", "k_trace", "k_shade_slots"]                   # round pipeline (large shallow frames)
+WAVE_CLASS_NAMES = ["-", "-", "k_wave", "-"]                                             # persistent wavefront (the other frames)
 COUNT_CLASS_NAMES = ["k_primary", "k_bounce_closest", "k_shadow", "k_shade"]             # counting wavefront (CGRT_RENDER_COUNT)
 
 

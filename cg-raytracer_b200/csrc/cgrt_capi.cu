@@ -248,6 +248,10 @@ struct WaveTuner {
     int next = 0, recording = -1;
 };
 
+// The kernel set that renders a frame (cgrt_kernels.h). The values are ABI: cgrt_render_stats::pipeline reports them and
+// capi.class_names and bench.py index by them.
+enum FramePipeline : uint32_t { PIPE_COUNT = 0, PIPE_PATHS = 1, PIPE_ROUNDS = 2, PIPE_WAVE = 3 };
+
 struct cgrt_scene {
     int device = 0;
     DeviceInfo di;
@@ -294,8 +298,8 @@ struct cgrt_scene {
     DevBuf<float4> waveResume;
     DevBuf<unsigned> waveLat;
     uint32_t waveSeq = 0;
-    int lastPipeline = 0; // 0 counting wavefront, 1 path pipeline, 2 round pipeline
-    int lastChains = 1;
+    FramePipeline lastPipeline = PIPE_COUNT; // kernel set of the last frame (choosePipeline)
+    int lastChains = 1;                      // PIPE_ROUNDS: chains of the last frame (their counters are summed)
     // streaming form (cgrt_render_submit / cgrt_render_wait)
     cudaStream_t copyStream = nullptr;
     cudaEvent_t renderDone[2] = {nullptr, nullptr}, copyDone[2] = {nullptr, nullptr};
@@ -306,10 +310,8 @@ struct cgrt_scene {
     uint64_t submitSeq = 0;
     int64_t fastStats[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     ChainSync chainSync{};
-    bool lastPathPipeline = false;
     std::vector<cudaEvent_t> traceEvents;
     WaveTrace trace{};
-    bool lastCounted = false;
     // tile partition of the current frame geometry (rebuilt only when width/height/tile/world/rank change)
     TileLayout layout;
     DevBuf<int2> tileSeq; // production order: (global tile id, local tile index), centre-out
@@ -1081,6 +1083,19 @@ static bool useWave(const cgrt_scene* s, const FrameParams& P)
     // 0.23 vs 0.37 ms, C5 on 4 GPUs 0.58 vs 0.64 ms - where the round pipeline's per-launch floors no longer shrink with the share)
     return pref == 1 || P.traceLimit >= 3 || P.nSlots < 400000 || (P.world > 1 && P.nSlots < 2500000);
 }
+
+// the one decision of which kernel set renders a frame: the counting wavefront when asked for, else the fastest the scene and
+// the frame allow
+static FramePipeline choosePipeline(const cgrt_scene* s, const FrameParams& P, int flags)
+{
+    if (flags & CGRT_RENDER_COUNT) return PIPE_COUNT;
+    if (useWave(s, P)) return PIPE_WAVE;
+    return useRounds(s, P) ? PIPE_ROUNDS : PIPE_PATHS;
+}
+// pipelines that keep hit records and depths per pixel slot (what the overlapped delivery of cgrt_render needs)
+static bool hasSlotRecords(FramePipeline pipe) { return pipe == PIPE_ROUNDS || pipe == PIPE_WAVE; }
+// independent sub-frames of the last frame, each with its own CGRT_CNT_TOTAL counters
+static int chainsOf(const cgrt_scene* s) { return s->lastPipeline == PIPE_ROUNDS ? s->lastChains : 1; }
 // tickets the queue must hold: every slot can cast one closest-hit ray and one shadow ray per light at every level; plus the
 // tickets idle lanes hold beyond the last ray (one per resident lane at most)
 static size_t waveTicketCap(const FrameParams& P)
@@ -1202,7 +1217,7 @@ static bool waveTuning(WaveQ& Q, int nSlots, int nLights, int world)
 }
 
 static int prepareFrame(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render_params* p, FrameParams& P,
-                        const int** dTileList, const int2** dTileSeq)
+                        const int** dTileList, const int2** dTileSeq, FramePipeline* pipe)
 {
     const int tw = p->tile_w > 0 ? p->tile_w : 8, th = p->tile_h > 0 ? p->tile_h : 8;
     const int key[6] = {p->width, p->height, tw, th, p->world, p->rank};
@@ -1257,15 +1272,21 @@ static int prepareFrame(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render
     const int nL = std::max(P.nLights, 1);
     const int levels = std::max(P.traceLimit - 1, 1);
     const int pathLevels = std::max(P.traceLimit, 1);
-    if (p->flags & CGRT_RENDER_COUNT) { // level-by-level counting pipeline
+    if (P.nSph > 0 && !useRounds(s, P)) return fail(CGRT_ERR_INVALID, "spherical lights need a scene with a search tree (not CGRT_SCENE_EXACT_ONLY / NO_SUBTREES)");
+    *pipe = choosePipeline(s, P, p->flags);
+    if (*pipe != PIPE_COUNT) { // hit records indexed by (pixel slot or path, level)
+        RC(s->hitRec.ensure(cap * pathLevels * 3));
+        RC(s->pathDepth.ensure(cap));
+        RC(s->lit.ensure(cap * pathLevels * nL));
+    }
+    switch (*pipe) {
+    case PIPE_COUNT: // level-by-level counting wavefront
         RC(s->hitQ.ensure(cap * 3));
         RC(s->bounceQ.ensure(cap * 2));
         RC(s->lit.ensure(cap * nL));
         RC(s->pathState.ensure(cap * 2 * levels));
-    } else if (useWave(s, P)) { // persistent wavefront: records indexed by (pixel slot, level), one ticket-indexed ray array
-        RC(s->hitRec.ensure(cap * pathLevels * 3));
-        RC(s->pathDepth.ensure(cap));
-        RC(s->lit.ensure(cap * pathLevels * nL));
+        break;
+    case PIPE_WAVE: { // persistent wavefront: one ticket-indexed ray array
         const size_t tickets = waveTicketCap(P);
         if (tickets >= ((size_t)1 << 30)) return fail(CGRT_ERR_INVALID, "frame too large for the ray queue's 30-bit tickets");
         if (!s->waveRays.p || s->waveRays.n < tickets * 3) { // (the records' tags compare against waveSeq >= 1: start from zero)
@@ -1277,10 +1298,9 @@ static int prepareFrame(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render
         }
         RC(s->waveCtl.ensure(WCTL_INTS));
         RC(s->waveResume.ensure((size_t)waveGridBlocks(s->di.numSMs) * 128 * WAVE_RESUME_F4));
-    } else if (useRounds(s, P)) { // round pipeline: records indexed by (pixel slot, level), two ray lists per kind
-        RC(s->hitRec.ensure(cap * pathLevels * 3));
-        RC(s->pathDepth.ensure(cap));
-        RC(s->lit.ensure(cap * pathLevels * nL));
+        break;
+    }
+    case PIPE_ROUNDS: { // round pipeline: two ray lists per kind
         if (P.nSph > 0) {
             RC(s->softList.ensure(cap * pathLevels + 1));
             RC(s->soft.ensure(cap * pathLevels * (size_t)P.nSph));
@@ -1292,21 +1312,20 @@ static int prepareFrame(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render
             RC(s->sRay[k].ensure(capR * nL * 3));
             RC(s->sRes[k].ensure(capR * nL));
         }
-    } else { // path pipeline: one record per (path, level)
-        RC(s->hitRec.ensure(cap * pathLevels * 3));
+        break;
+    }
+    case PIPE_PATHS: // path pipeline: compacted list of the records
         RC(s->hitList.ensure(cap * pathLevels));
-        RC(s->pathDepth.ensure(cap));
-        RC(s->lit.ensure(cap * pathLevels * nL));
         if (s->dev.fastRoot != 0u) { // replay queues of the speculative kernels
             RC(s->replayQ.ensure(cap * 3));
             RC(s->replayShadow.ensure(cap * pathLevels * nL));
         }
+        break;
     }
     RC(s->pathPix.ensure(cap));
     RC(s->counts.ensure(CGRT_CNT_TOTAL * CGRT_MAX_CHAINS));
     RC(s->tests.ensure(6));
     // parameter block: FrameParams header + lights (2 x float4 each)
-    if (P.nSph > 0 && !useRounds(s, P)) return fail(CGRT_ERR_INVALID, "spherical lights need a scene with a search tree (not CGRT_SCENE_EXACT_ONLY / NO_SUBTREES)");
     const size_t need = CGRT_PARAM_BLOCK_HEADER + ((size_t)nL + (size_t)P.nSph) * 32;
     if (need > s->paramBlockBytes || !s->hParamRing) {
         CK(cudaDeviceSynchronize());
@@ -1328,6 +1347,88 @@ int cgrt_bvh_fast_tree_stats(const cgrt_scene* s, int64_t* out)
     return CGRT_OK;
 }
 
+// ---- each pipeline's view of the scene's frame buffers (sized by prepareFrame) ---------------------------------------------------
+static CountBuffers countBuffers(const cgrt_scene* s, const FrameParams& P)
+{
+    CountBuffers B;
+    B.hitQ = s->hitQ.p;
+    B.bounceQ = s->bounceQ.p;
+    B.lit = s->lit.p;
+    B.pathPix = s->pathPix.p;
+    B.pathState = s->pathState.p;
+    B.counts = s->counts.p;
+    B.tests = s->tests.p;
+    B.cap = (size_t)std::max(P.nSlots, 1);
+    return B;
+}
+
+static PathBuffers pathBuffers(const cgrt_scene* s, const FrameParams& P)
+{
+    PathBuffers B;
+    B.hitRec = s->hitRec.p;
+    B.hitList = s->hitList.p;
+    B.lit = s->lit.p;
+    B.pathPix = s->pathPix.p;
+    B.pathDepth = s->pathDepth.p;
+    B.replayQ = s->replayQ.p;
+    B.replayShadow = s->replayShadow.p;
+    B.counts = s->counts.p;
+    B.cap = (size_t)std::max(P.nSlots, 1);
+    B.levels = std::max(P.traceLimit, 1);
+    return B;
+}
+
+// chain c of nChains: its own ray lists and counters, the frame's hit records
+static RoundBuffers roundBuffers(const cgrt_scene* s, const FrameParams& P, int c, int nChains)
+{
+    const size_t tpx = (size_t)P.tileW * P.tileH;
+    const size_t capC = ((size_t)std::max(P.nSlots, 1) / tpx / nChains + 1) * tpx; // slots one chain can own
+    const size_t nLc = (size_t)std::max(P.nLights, 1);
+    RoundBuffers B;
+    for (int k = 0; k < 2; k++) {
+        B.cRay[k] = s->cRay[k].p + c * capC * 3; B.cRes[k] = s->cRes[k].p + c * capC;
+        B.sRay[k] = s->sRay[k].p + c * capC * nLc * 3; B.sRes[k] = s->sRes[k].p + c * capC * nLc;
+    }
+    B.hitRec = s->hitRec.p;
+    B.lit = s->lit.p;
+    B.pathDepth = s->pathDepth.p;
+    B.counts = s->counts.p + c * CGRT_CNT_TOTAL;
+    B.levels = std::max(P.traceLimit, 1);
+    B.softList = s->softList.p;
+    B.soft = s->soft.p;
+    B.softSeed = s->softSeed;
+    return B;
+}
+
+// k_wave's ray / finish queues (its records and counters are those of a one-chain round frame). Clears the optional
+// diagnostics buffers on `st`.
+static int waveQueues(cgrt_scene* s, cudaStream_t st, WaveQ& Q)
+{
+    Q.rays = s->waveRays.p;
+    Q.fin = s->waveFin.p;
+    Q.ctl = s->waveCtl.p;
+    Q.seq = ++s->waveSeq;
+    if (Q.seq == 0u) Q.seq = ++s->waveSeq;
+    Q.cap = (int)std::min<size_t>(s->waveRays.n / 3, (size_t)0x3fffffff);
+    Q.resume = s->waveResume.p;
+    Q.resumeCap = (int)std::min<size_t>(s->waveResume.n / WAVE_RESUME_F4, (size_t)0xffffff);
+    Q.lat = nullptr;
+#ifdef CGRT_WAVE_LAT
+    if (getenv("CGRT_WAVE_LAT")) {
+        RC(s->waveLat.ensure((size_t)Q.cap * 16));
+        CK(cudaMemsetAsync(s->waveLat.p, 0, (size_t)Q.cap * 16 * sizeof(unsigned), st));
+        Q.lat = s->waveLat.p;
+    }
+#endif
+    Q.trace = nullptr;
+    if (getenv("CGRT_WAVE_TRACE") || Q.lat != nullptr) { // timeline of the frame's counters (cgrt_debug_wave_timeline); off by default
+        RC(s->waveTrace.ensure((size_t)WAVE_TRACE_SAMPLES * 8));
+        CK(cudaMemsetAsync(s->waveTrace.p, 0, (size_t)WAVE_TRACE_SAMPLES * 8 * sizeof(int), st));
+        Q.trace = s->waveTrace.p;
+    }
+    return CGRT_OK;
+}
+
 int cgrt_render_device(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render_params* p, float* d_out, void* stream)
 {
     if (!s || !cam || !d_out) return fail(CGRT_ERR_INVALID, "null argument");
@@ -1338,8 +1439,9 @@ int cgrt_render_device(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render_
     FrameParams P;
     const int* dTiles = nullptr;
     const int2* dSeq = nullptr;
-    RC(prepareFrame(s, cam, p, P, &dTiles, &dSeq));
-    if (P.screenLayout && P.world > 1 && (p->flags & CGRT_RENDER_COUNT))
+    FramePipeline pipe;
+    RC(prepareFrame(s, cam, p, P, &dTiles, &dSeq, &pipe));
+    if (P.screenLayout && P.world > 1 && pipe == PIPE_COUNT)
         return fail(CGRT_ERR_INVALID, "CGRT_RENDER_COUNT renders into the tile-major buffer; it cannot be combined with CGRT_RENDER_SCREEN_LAYOUT");
     // per-frame upload (camera constants + lights, read live from the scene like src/main.cpp:835-876 allows)
     unsigned char* slot = s->hParamRing + (size_t)s->ringPos * s->paramBlockBytes;
@@ -1358,15 +1460,6 @@ int cgrt_render_device(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render_
     }
     const size_t bytes = CGRT_PARAM_BLOCK_HEADER + (s->lights.size() + (size_t)P.nSph) * 32;
     CK(cudaMemcpyAsync(s->dParamBlock.p, slot, bytes, cudaMemcpyHostToDevice, st));
-    WaveBuffers B;
-    B.hitQ = s->hitQ.p;
-    B.bounceQ = s->bounceQ.p;
-    B.lit = s->lit.p;
-    B.pathPix = s->pathPix.p;
-    B.pathState = s->pathState.p;
-    B.counts = s->counts.p;
-    B.tests = s->tests.p;
-    B.cap = (size_t)std::max(P.nSlots, 1);
     const int maxKernels = CGRT_TRACE_MAX_KERNELS;
     if ((p->flags & CGRT_RENDER_PROFILE_ALL) && s->traceEvents.empty()) {
         s->traceEvents.resize(2 * maxKernels);
@@ -1376,60 +1469,19 @@ int cgrt_render_device(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render_
     s->trace.ev = s->traceEvents.data();
     s->trace.maxKernels = maxKernels;
     s->trace.classMask = p->flags & CGRT_RENDER_PROFILE_ALL;
-    const bool countTests = (p->flags & CGRT_RENDER_COUNT) != 0;
+    const FrameParams* dP = (const FrameParams*)s->dParamBlock.p;
+    const float4* dLights = (const float4*)(s->dParamBlock.p + CGRT_PARAM_BLOCK_HEADER);
+    const int numSMs = s->di.numSMs;
     CK(cudaEventRecord(s->ev0, st));
-    int launches;
-    if (countTests) {
-        launches = launchWavefront(s->dev, (const FrameParams*)s->dParamBlock.p, P,
-                                   (const float4*)(s->dParamBlock.p + CGRT_PARAM_BLOCK_HEADER), B, dTiles, d_out,
-                                   s->di.numSMs, true, &s->trace, st);
-    } else if (useWave(s, P)) {
-        RoundBuffers RB;
-        for (int k = 0; k < 2; k++) { RB.cRay[k] = nullptr; RB.cRes[k] = nullptr; RB.sRay[k] = nullptr; RB.sRes[k] = nullptr; }
-        RB.hitRec = s->hitRec.p;
-        RB.lit = s->lit.p;
-        RB.pathDepth = s->pathDepth.p;
-        RB.counts = s->counts.p;
-        RB.levels = std::max(P.traceLimit, 1);
-        RB.softList = nullptr;
-        RB.soft = nullptr;
-        RB.softSeed = 0u;
-        WaveQ Q;
-        Q.rays = s->waveRays.p;
-        Q.fin = s->waveFin.p;
-        Q.ctl = s->waveCtl.p;
-        Q.seq = ++s->waveSeq;
-        if (Q.seq == 0u) Q.seq = ++s->waveSeq;
-        Q.cap = (int)std::min<size_t>(s->waveRays.n / 3, (size_t)0x3fffffff);
-        Q.resume = s->waveResume.p;
-        Q.resumeCap = (int)std::min<size_t>(s->waveResume.n / WAVE_RESUME_F4, (size_t)0xffffff);
-        Q.lat = nullptr;
-#ifdef CGRT_WAVE_LAT
-        if (getenv("CGRT_WAVE_LAT")) {
-            RC(s->waveLat.ensure((size_t)Q.cap * 16));
-            CK(cudaMemsetAsync(s->waveLat.p, 0, (size_t)Q.cap * 16 * sizeof(unsigned), st));
-            Q.lat = s->waveLat.p;
-        }
-#endif
-        Q.trace = nullptr;
-        if (getenv("CGRT_WAVE_TRACE") || Q.lat != nullptr) { // timeline of the frame's counters (cgrt_debug_wave_timeline); off by default
-            RC(s->waveTrace.ensure((size_t)WAVE_TRACE_SAMPLES * 8));
-            CK(cudaMemsetAsync(s->waveTrace.p, 0, (size_t)WAVE_TRACE_SAMPLES * 8 * sizeof(int), st));
-            Q.trace = s->waveTrace.p;
-        }
-        const bool tuned = waveTuning(Q, P.nSlots, P.nLights, P.world) && !(p->flags & CGRT_RENDER_PROFILE_ALL);
-        if (tuned) {
-            const int key[8] = {P.width, P.height, P.nSlots, P.traceLimit, P.nLights, P.world, P.rank, Q.mode};
-            Q.finEvery = waveTunerChoose(s->tuner, key, Q.finEvery);
-            waveTunerBegin(s->tuner, Q.finEvery, st);
-        }
-        launches = launchWavePipeline(s->dev, (const FrameParams*)s->dParamBlock.p, P,
-                                      (const float4*)(s->dParamBlock.p + CGRT_PARAM_BLOCK_HEADER), RB, Q, dSeq, d_out,
-                                      s->di.numSMs, &s->trace, st);
-        if (tuned) waveTunerEnd(s->tuner, st);
-        s->lastChains = 1;
-        s->lastPipeline = 3;
-    } else if (useRounds(s, P)) {
+    int launches = 0;
+    switch (pipe) {
+    case PIPE_COUNT:
+        launches = launchCountingFrame(s->dev, dP, P, dLights, countBuffers(s, P), dTiles, d_out, numSMs, &s->trace, st);
+        break;
+    case PIPE_PATHS:
+        launches = launchPathPipeline(s->dev, dP, P, dLights, pathBuffers(s, P), dSeq, d_out, numSMs, &s->trace, st);
+        break;
+    case PIPE_ROUNDS: {
         // chains: independent sub-frames (tiles dealt round-robin) on their own streams
         const int nChains = roundPipelineChains(P.nSlots);
         if (nChains > 1 && !s->chainSync.fork) {
@@ -1440,49 +1492,27 @@ int cgrt_render_device(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render_
             }
         }
         RoundBuffers RB[CGRT_MAX_CHAINS];
-        const size_t tpx = (size_t)P.tileW * P.tileH;
-        const size_t capC = ((size_t)std::max(P.nSlots, 1) / tpx / nChains + 1) * tpx; // slots one chain can own
-        const size_t nLc = (size_t)std::max(P.nLights, 1);
-        for (int c = 0; c < nChains; c++) {
-            for (int k = 0; k < 2; k++) {
-                RB[c].cRay[k] = s->cRay[k].p + c * capC * 3; RB[c].cRes[k] = s->cRes[k].p + c * capC;
-                RB[c].sRay[k] = s->sRay[k].p + c * capC * nLc * 3; RB[c].sRes[k] = s->sRes[k].p + c * capC * nLc;
-            }
-            RB[c].hitRec = s->hitRec.p;
-            RB[c].lit = s->lit.p;
-            RB[c].pathDepth = s->pathDepth.p;
-            RB[c].counts = s->counts.p + c * CGRT_CNT_TOTAL;
-            RB[c].levels = std::max(P.traceLimit, 1);
-            RB[c].softList = s->softList.p;
-            RB[c].soft = s->soft.p;
-            RB[c].softSeed = s->softSeed;
-        }
-        launches = launchRoundPipeline(s->dev, (const FrameParams*)s->dParamBlock.p, P,
-                                       (const float4*)(s->dParamBlock.p + CGRT_PARAM_BLOCK_HEADER), RB, nChains, s->chainSync,
-                                       dSeq, d_out, s->di.numSMs, &s->trace, st);
+        for (int c = 0; c < nChains; c++) RB[c] = roundBuffers(s, P, c, nChains);
+        launches = launchRoundPipeline(s->dev, dP, P, dLights, RB, nChains, s->chainSync, dSeq, d_out, numSMs, &s->trace, st);
         s->lastChains = nChains;
-        s->lastPipeline = 2;
-    } else {
-        s->lastPipeline = 1;
-        PathBuffers PB;
-        PB.hitRec = s->hitRec.p;
-        PB.hitList = s->hitList.p;
-        PB.lit = s->lit.p;
-        PB.pathPix = s->pathPix.p;
-        PB.pathDepth = s->pathDepth.p;
-        PB.replayQ = s->replayQ.p;
-        PB.replayShadow = s->replayShadow.p;
-        PB.counts = s->counts.p;
-        PB.cap = B.cap;
-        PB.levels = std::max(P.traceLimit, 1);
-        launches = launchPathPipeline(s->dev, (const FrameParams*)s->dParamBlock.p, P,
-                                      (const float4*)(s->dParamBlock.p + CGRT_PARAM_BLOCK_HEADER), PB, dSeq, d_out,
-                                      s->di.numSMs, &s->trace, st);
+        break;
     }
-    s->lastPathPipeline = !countTests;
-    if (countTests) s->lastPipeline = 0;
+    case PIPE_WAVE: {
+        WaveQ Q;
+        RC(waveQueues(s, st, Q));
+        const bool tuned = waveTuning(Q, P.nSlots, P.nLights, P.world) && !(p->flags & CGRT_RENDER_PROFILE_ALL);
+        if (tuned) {
+            const int key[8] = {P.width, P.height, P.nSlots, P.traceLimit, P.nLights, P.world, P.rank, Q.mode};
+            Q.finEvery = waveTunerChoose(s->tuner, key, Q.finEvery);
+            waveTunerBegin(s->tuner, Q.finEvery, st);
+        }
+        launches = launchWavePipeline(s->dev, dP, P, dLights, roundBuffers(s, P, 0, 1), Q, dSeq, d_out, numSMs, &s->trace, st);
+        if (tuned) waveTunerEnd(s->tuner, st);
+        break;
+    }
+    }
+    s->lastPipeline = pipe;
     CK(cudaEventRecord(s->ev1, st));
-    s->lastCounted = countTests;
     CK(cudaGetLastError());
     s->lastStream = st;
     s->statsOnHost = false;
@@ -1503,7 +1533,7 @@ int cgrt_render_collect_stats(cgrt_scene* s, cgrt_render_stats* stats)
     int counts[CGRT_CNT_TOTAL];
     const bool onHost = s->statsOnHost && s->hStats != nullptr;
     {
-        const int nc = s->lastPipeline == 2 ? s->lastChains : 1;
+        const int nc = chainsOf(s);
         std::vector<int> all((size_t)CGRT_CNT_TOTAL * nc);
         if (onHost) std::memcpy(all.data(), s->hStats, all.size() * sizeof(int));
         else CK(cudaMemcpy(all.data(), s->counts.p, all.size() * sizeof(int), cudaMemcpyDeviceToHost));
@@ -1516,14 +1546,14 @@ int cgrt_render_collect_stats(cgrt_scene* s, cgrt_render_stats* stats)
     // logical rays (SURVEY.md §8(d)): primary = pixels of this rank inside the image
     const uint64_t primary = s->primaryPixels;
     stats->primary = primary;
-    if (s->lastPipeline == 3) { // persistent wavefront: the watchdog of k_wave (a warp waited for seconds) invalidates the frame
+    if (s->lastPipeline == PIPE_WAVE) { // persistent wavefront: the watchdog of k_wave (a warp waited for seconds) invalidates the frame
         int err = 0;
         if (onHost) err = s->hStats[CGRT_CNT_TOTAL * CGRT_MAX_CHAINS];
         else CK(cudaMemcpy(&err, s->waveCtl.p + WCTL_ERR, sizeof(int), cudaMemcpyDeviceToHost));
         if (err) return fail(CGRT_ERR_CUDA, "k_wave watchdog: the persistent wavefront did not complete; the frame is invalid");
     }
-    stats->pipeline = (uint32_t)s->lastPipeline;
-    if (s->lastPipeline == 2 || s->lastPipeline == 3) {
+    stats->pipeline = s->lastPipeline;
+    if (hasSlotRecords(s->lastPipeline)) {
         stats->primary_hit = (uint64_t)counts[CGRT_CNT_PATHS];
         for (int l = 0; l < P.traceLimit; l++) {
             stats->shadow += (uint64_t)counts[CGRT_CNT_HIT + l] * (uint64_t)P.nLights;
@@ -1536,13 +1566,13 @@ int cgrt_render_collect_stats(cgrt_scene* s, cgrt_render_stats* stats)
         }
         stats->replayed_closest = (uint32_t)counts[CGRT_CNT_REPLAY_PATHS];
         stats->replayed_shadow = (uint32_t)counts[CGRT_CNT_REPLAY_SHADOW];
-    } else if (s->lastPathPipeline) {
+    } else if (s->lastPipeline == PIPE_PATHS) {
         stats->primary_hit = (uint64_t)counts[CGRT_CNT_PATHS];
         stats->shadow = (uint64_t)counts[CGRT_CNT_HITS] * (uint64_t)P.nLights;
         stats->bounce = (uint64_t)counts[CGRT_CNT_BOUNCES];
         stats->replayed_closest = (uint32_t)counts[CGRT_CNT_REPLAY_PATHS];
         stats->replayed_shadow = (uint32_t)counts[CGRT_CNT_REPLAY_SHADOW];
-    } else {
+    } else { // PIPE_COUNT
         stats->primary_hit = (uint64_t)counts[CGRT_CNT_HIT + 0];
         for (int l = 0; l < P.traceLimit; l++) {
             stats->shadow += (uint64_t)counts[CGRT_CNT_HIT + l] * (uint64_t)P.nLights;
@@ -1583,7 +1613,7 @@ int cgrt_render_collect_stats(cgrt_scene* s, cgrt_render_stats* stats)
             stats->class_ms[c] = total;
         }
     }
-    if (s->lastCounted) {
+    if (s->lastPipeline == PIPE_COUNT) {
         unsigned long long t[6];
         CK(cudaMemcpy(t, s->tests.p, sizeof t, cudaMemcpyDeviceToHost));
         for (int c = 0; c < 3; c++) {
@@ -1642,7 +1672,7 @@ int cgrt_render(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render_params*
         overlapped = true;
     }
     RC(cgrt_render_device(s, cam, p, s->frame.p, s->stream));
-    if (overlapped && !(s->lastPipeline == 2 || s->lastPipeline == 3)) { // (path pipeline: no per-slot depth) plain copy after all
+    if (overlapped && !hasSlotRecords(s->lastPipeline)) { // (path pipeline: no per-slot depth) plain copy after all
         CK(cudaStreamSynchronize(s->copyStream));
         overlapped = false;
     }
@@ -1658,10 +1688,9 @@ int cgrt_render(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render_params*
                 cudaGetLastError();
             }
             if (s->hStats) {
-                const int nc = s->lastPipeline == 2 ? s->lastChains : 1;
-                CK(cudaMemcpyAsync(s->hStats, s->counts.p, sizeof(int) * CGRT_CNT_TOTAL * nc, cudaMemcpyDeviceToHost, s->stream));
+                CK(cudaMemcpyAsync(s->hStats, s->counts.p, sizeof(int) * CGRT_CNT_TOTAL * chainsOf(s), cudaMemcpyDeviceToHost, s->stream));
                 s->hStats[CGRT_CNT_TOTAL * CGRT_MAX_CHAINS] = 0;
-                if (s->lastPipeline == 3)
+                if (s->lastPipeline == PIPE_WAVE)
                     CK(cudaMemcpyAsync(s->hStats + CGRT_CNT_TOTAL * CGRT_MAX_CHAINS, s->waveCtl.p + WCTL_ERR, sizeof(int), cudaMemcpyDeviceToHost, s->stream));
                 fetched = true;
             }

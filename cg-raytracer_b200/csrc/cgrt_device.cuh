@@ -109,16 +109,6 @@ RT_DEV bool leafCandidate(const DevScene& S, int i, const V3& o, const V3& d, Le
 
 #define CGRT_WIDE_STRIDE 16 // float4 per 8-wide node: 14 used, padded to 256 B = exactly two 128-byte lines
 
-// L1 prefetch hint: starts the fetch of a line the next step will read, without tying up a register
-RT_DEV void prefetchL1(const void* p)
-{
-#ifdef __CUDA_ARCH__
-    asm volatile("prefetch.global.L1 [%0];" ::"l"(p));
-#else
-    (void)p; // (this header is also compiled for the host by tests/spec_harness.cpp)
-#endif
-}
-
 #define CGRT_RHO 1e-6f
 #define CGRT_TAU 1e-30f
 RT_DEV float errBound(float x) { return fabsf(x) * CGRT_RHO + CGRT_TAU; }
@@ -516,16 +506,11 @@ struct FastTrav {
 // triangle closer than t* (1 + 1e-6) (the pruning of the search uses the same factor)
 #define CGRT_NEAR 1.000001f
 #define CGRT_FASTSTACK 64
-#ifndef CGRT_PREFETCH
-#define CGRT_PREFETCH 0 // measured slower on B200 (k_trace 1.82 -> 2.08 ms/frame): the steps are issue-bound, not fetch-bound
-#endif
 struct FastStack {
     uint2 e[CGRT_FASTSTACK]; // (node id, entry distance): one 8-byte local-memory access per push / pop
     float t2; // smallest distance of any OTHER acceptable triangle met so far (runner-up), +inf none: see certifyClosest. Lives
               // here (local memory) because it is touched only when a candidate is accepted; a register in the hot loop is not
 };
-
-RT_DEV void fastPrefetch(const DevScene& S, uint32_t id);
 
 // intersectDataStructure (bvh.cpp:831-844) evaluated exactly, then the fast tree's root.
 // TRAV_DONE: the reference does not enter the tree (certain miss); TRAV_DEFER: this ray must take the exact traversal.
@@ -557,34 +542,16 @@ RT_DEV int fastBegin(const DevScene& S, FastTrav& T, const V3& o, const V3& d, f
     T.inv.y = ay == 0.0f ? 1e30f : 1.0f / d.y;
     T.inv.z = az == 0.0f ? 1e30f : 1.0f / d.z;
     T.node = S.fastRoot;
-    fastPrefetch(S, T.node);
     return TRAV_CONTINUE;
 }
 
-// start fetching what the next step on `id` reads: both lines of an 8-wide node, or the 64-byte records of a leaf's triangles
-RT_DEV void fastPrefetch(const DevScene& S, uint32_t id)
-{
-#if CGRT_PREFETCH
-    if (id & CGRT_TRI) {
-        const float4* tr = S.tri4f + 4 * (size_t)(id & CGRT_IDX_MASK);
-        const int count = (int)((id >> CGRT_TRICNT_SHIFT) & 7u) + 1;
-        for (int k = 0; k < count; k++) prefetchL1(tr + 4 * k);
-    } else {
-        const float4* w = S.wide + CGRT_WIDE_STRIDE * (size_t)(id & CGRT_IDX_MASK);
-        prefetchL1(w);
-        prefetchL1(w + 8);
-    }
-#endif
-}
-
-RT_DEV int fastPop(const DevScene& S, FastTrav& T, FastStack& K, float bound)
+RT_DEV int fastPop(FastTrav& T, FastStack& K, float bound)
 {
     while (T.sp > 0) {
         T.sp--;
         const uint2 e = K.e[T.sp];
         if (__uint_as_float(e.y) > bound) continue;
         T.node = e.x;
-        fastPrefetch(S, T.node);
         return TRAV_CONTINUE;
     }
     return TRAV_DONE;
@@ -629,7 +596,7 @@ RT_DEV int fastStepWideDyn(const DevScene& S, FastTrav& T, FastStack& K, bool an
             if (hit) hitMask |= 1u << (4 * h + c);
         }
     }
-    if (hitMask == 0u) return fastPop(S, T, K, bt);
+    if (hitMask == 0u) return fastPop(T, K, bt);
     if (T.sp + 7 > CGRT_FASTSTACK) return TRAV_DEFER; // pathological depth: let the exact traversal handle the ray
     int best = -1;
     float bestT = 0.0f;
@@ -645,7 +612,6 @@ RT_DEV int fastStepWideDyn(const DevScene& S, FastTrav& T, FastStack& K, bool an
         }
     }
     T.node = cid[best];
-    fastPrefetch(S, T.node);
     return TRAV_CONTINUE;
 }
 template <bool ANY>
@@ -736,7 +702,7 @@ RT_DEV int fastStepLeafDyn(const DevScene& S, FastTrav& T, FastStack& K, bool an
         if (any && !(tt + eps >= maxDist)) return TRAV_FIRED;
     }
     // search bound: fminf(t, maxDist) for shadow rays; closest-hit rays carry maxDist = +inf or are bounded by t alone
-    return fastPop(S, T, K, (any ? fminf(T.t, maxDist) : T.t) * 1.000001f);
+    return fastPop(T, K, (any ? fminf(T.t, maxDist) : T.t) * 1.000001f);
 }
 template <bool ANY>
 RT_DEV int fastStepLeaf(const DevScene& S, FastTrav& T, FastStack& K, float eps, float maxDist)

@@ -91,19 +91,25 @@ struct FrameParams {
     int nSph;               // spherical lights (2 x float4 each, after the point lights in the parameter block)
 };
 
-// Queues of the wavefront (all sized for the worst case `cap` = nSlots; only the used prefix is ever touched).
-struct WaveBuffers {
+// Four kernel sets render a frame; cgrt_capi.cu choosePipeline picks one per frame (all give the same pixels and ray counts):
+//   counting wavefront  CGRT_RENDER_COUNT                                         launchCountingFrame, CountBuffers
+//   path pipeline       scenes without a fast tree; frames too large for rounds   launchPathPipeline, PathBuffers
+//   round pipeline      large shallow frames of scenes with a fast tree           launchRoundPipeline, RoundBuffers per chain
+//   k_wave              every other frame of a scene with a fast tree             launchWavePipeline, RoundBuffers + WaveQ
+
+// Queues of the counting wavefront (all sized for the worst case `cap` = nSlots; only the used prefix is ever touched).
+struct CountBuffers {
     float4* hitQ;      // 3 x float4 per hit:   [P | matId] [N | outIdx] [D | pathId]
     float4* bounceQ;   // 2 x float4 per ray:   [origin | tmax] [direction | pathId]
     uint8_t* lit;      // [hit][light] 1 = light reaches the point
     int* pathPix;      // [pathId] output index of the path's pixel
     float4* pathState; // [level][pathId] 2 x float4: directColor, ks of the shade() frame waiting for its reflection
     int* counts;       // CGRT_CNT_TOTAL queue lengths
-    unsigned long long* tests; // [class 0..2][box, tri] reference test counts (counting variants only)
+    unsigned long long* tests; // [class 0..2][box, tri] reference test counts
     size_t cap;
 };
 
-// Queues of the production pipeline (cgrt_kernels.cu "path pipeline"): one persistent closest-hit kernel follows every
+// Queues of the path pipeline (cgrt_kernels.cu "path pipeline"): one persistent closest-hit kernel follows every
 // path from its primary ray through its mirror bounces and leaves one hit record per (path, level); all shadow rays of the
 // frame are then traced by one any-hit launch and one shading launch folds each path back to its pixel.
 struct PathBuffers {
@@ -114,12 +120,12 @@ struct PathBuffers {
     int* pathDepth;    // [path] number of levels that recorded a hit
     float4* replayQ;   // 3 x float4 per deferred ray: [origin | tmax] [direction | level] [path, outIdx, -, -]
     int* replayShadow; // deferred shadow work items (index of the lit flag)
-    int* counts;       // shared with WaveBuffers::counts
+    int* counts;       // shared with CountBuffers::counts
     size_t cap;        // paths the buffers can hold (= local pixel slots)
     int levels;        // trace limit the buffers are laid out for
 };
 
-// Buffers of the ROUND pipeline (production when the scene has a fast tree; cgrt_kernels.cu "round pipeline"):
+// Buffers of the ROUND pipeline (cgrt_kernels.cu "round pipeline"; k_wave uses the records and counters, not the ray lists):
 //   k_gen      : one thread per pixel slot: primary ray, the reference's root-box test, compacted list of rays that enter
 //   round r    : k_trace  - persistent warps, speculative search ONLY (no prologue / epilogue code in the hot loop) over the
 //                           closest-hit rays of level r and the shadow rays of the hits of level r-1
@@ -206,9 +212,9 @@ void launchUnitTrianglePlane(const float* tris, size_t n, float4* planes, cudaSt
 void launchUnitPointInTriangle(const float* in, size_t n, uint8_t* inside, cudaStream_t st);
 void launchUnitSphere(const float4* spheres, const float4* rays, size_t n, float* out, cudaStream_t st);
 void launchGenerateRays(const FrameParams* dP, int nPixels, float4* rays, cudaStream_t st);
-int launchWavefront(const DevScene& S, const FrameParams* dP, const FrameParams& hP, const float4* dLights,
-                    const WaveBuffers& B, const int* dTileList, float* fb, int numSMs, bool countTests, WaveTrace* tr,
-                    cudaStream_t st);
+// The launchers return the kernels they launched (cgrt_render_stats::kernel_launches).
+int launchCountingFrame(const DevScene& S, const FrameParams* dP, const FrameParams& hP, const float4* dLights,
+                        const CountBuffers& B, const int* dTileList, float* fb, int numSMs, WaveTrace* tr, cudaStream_t st);
 int launchPathPipeline(const DevScene& S, const FrameParams* dP, const FrameParams& hP, const float4* dLights,
                        const PathBuffers& B, const int2* dTileSeq, float* fb, int numSMs, WaveTrace* tr, cudaStream_t st);
 #define CGRT_MAX_CHAINS 8
@@ -222,7 +228,7 @@ int launchRoundPipeline(const DevScene& S, const FrameParams* dP, const FramePar
                         const RoundBuffers* chains, int nChains, const ChainSync& sync, const int2* dTileSeq, float* fb,
                         int numSMs, WaveTrace* tr, cudaStream_t st);
 // one kernel per frame: phase A ray generation, phase B search + finish over the device-side queue, phase C shading
-int waveGridBlocks(int numSMs); // co-resident CTAs of k_wave on this device (occupancy x SMs; CGRT_TUNE blocks=N caps the per-SM count)
+int waveGridBlocks(int numSMs); // co-resident CTAs of k_wave on this device (occupancy x SMs; CGRT_TUNE waveblocks=N caps the per-SM count)
 int launchWavePipeline(const DevScene& S, const FrameParams* dP, const FrameParams& hP, const float4* dLights,
                        const RoundBuffers& B, const WaveQ& Q, const int2* dTileSeq, float* fb, int numSMs, WaveTrace* tr,
                        cudaStream_t st);

@@ -652,7 +652,7 @@ RT_DEV bool waveLaneLoop(const DevScene& S, const WaveQ& Q, unsigned long long t
             const int sLeaf = __popc(__ballot_sync(0xffffffffu, leaf));
             const int nDone = __popc(__ballot_sync(0xffffffffu, st == WS_RUN && state != TRAV_CONTINUE));
             if (sAll == 0 || (nDone >= CGRT_WAVE_REFILL && it > 0)) break;
-            if (sAll - sLeaf >= sLeaf * CGRT_FAST_W_LEAF) {
+            if (sAll - sLeaf >= sLeaf) {
                 if (run && !leaf) state = fastStepWideDyn(S, T, K, any, maxDist);
             } else {
                 if (leaf) state = fastStepLeafDyn(S, T, K, any, eps, maxDist);

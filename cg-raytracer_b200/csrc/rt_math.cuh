@@ -8,15 +8,6 @@
 #include <stdint.h>
 
 #define RT_DEV __device__ __forceinline__
-// rarely executed helpers (exact fallbacks, the fp64 hit epilogue): out of line keeps the hot traversal loop small
-#ifndef CGRT_NOINLINE_RARE
-#define CGRT_NOINLINE_RARE 0 // measured slower on B200 (ABI spills outweigh the smaller loop), profiles/r01_tuning.md
-#endif
-#if CGRT_NOINLINE_RARE
-#define CGRT_RARE __device__ __noinline__
-#else
-#define CGRT_RARE __device__ __forceinline__
-#endif
 
 struct V3 {
     float x, y, z;
@@ -129,9 +120,9 @@ RT_DEV float areaDev(const V3& a, const V3& b, const V3& c)
 // ---- accepted-hit epilogue of intersectRayWithTriangle  src/ray_tracing.cpp:92-107 ---------------------------------------
 // The reference evaluates this for every accepted candidate; only the last accepted one survives, so the wavefront
 // evaluates it once for the final hit (same inputs -> same bits).
-CGRT_RARE void hitEpilogue(const V3& v0, const V3& v1, const V3& v2, const V3& n0, const V3& n1, const V3& n2,
-                        const V3& planeN, const V3& o, const V3& d, float t, float& alpha, float& beta, float& gamma,
-                        V3& normal)
+RT_DEV void hitEpilogue(const V3& v0, const V3& v1, const V3& v2, const V3& n0, const V3& n1, const V3& n2,
+                     const V3& planeN, const V3& o, const V3& d, float t, float& alpha, float& beta, float& gamma,
+                     V3& normal)
 {
     const V3 p = o + d * t;
     const float whole = areaDev(v0, v1, v2);
