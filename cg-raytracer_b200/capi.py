@@ -79,6 +79,7 @@ EXPORTS = [
     "cgrt_memset_device", "cgrt_memcpy_d2h_async", "cgrt_peer_export", "cgrt_peer_open", "cgrt_peer_close",
     "cgrt_flag_signal", "cgrt_flag_wait", "cgrt_bvh_fast_tree_stats", "cgrt_render_submit", "cgrt_render_wait",
     "cgrt_render_effects", "cgrt_scene_set_spherical_lights", "cgrt_debug_wave_timeline", "cgrt_debug_wave_tuner",
+    "cgrt_render_views", "cgrt_render_views_device",
 ]
 
 _lib = None
@@ -126,6 +127,8 @@ def load_library(path=None):
         "cgrt_generate_rays": (C.c_int, [C.c_int, C.POINTER(Camera), i32, i32, vp]),
         "cgrt_render": (C.c_int, [vp, C.POINTER(Camera), C.POINTER(RenderParams), vp, C.POINTER(RenderStats)]),
         "cgrt_render_device": (C.c_int, [vp, C.POINTER(Camera), C.POINTER(RenderParams), vp, vp]),
+        "cgrt_render_views": (C.c_int, [vp, C.POINTER(Camera), i32, C.POINTER(RenderParams), vp, C.POINTER(RenderStats)]),
+        "cgrt_render_views_device": (C.c_int, [vp, C.POINTER(Camera), i32, C.POINTER(RenderParams), vp, vp]),
         "cgrt_render_collect_stats": (C.c_int, [vp, C.POINTER(RenderStats)]),
         "cgrt_tile_buffer_floats": (sz, [C.POINTER(RenderParams)]),
         "cgrt_tile_list": (C.c_int, [C.POINTER(RenderParams), i32, i32p, i32]),
@@ -352,6 +355,21 @@ class Scene:
 
     def render_device(self, cam, params, d_out_ptr, stream_ptr=0):
         check(self.lib.cgrt_render_device(self.h, C.byref(cam), C.byref(params), C.c_void_p(d_out_ptr), C.c_void_p(stream_ptr)))
+
+    def render_views(self, cams, W, H, trace_limit=2, flags=0):
+        """Several cameras of this scene in one frame (cgrt_render_views): (rgb[K,H,W,3], stats dict summed over the views)."""
+        arr = (Camera * len(cams))(*cams)
+        p = render_params(W, H, trace_limit, flags=flags)
+        rgb = np.zeros((len(cams), H, W, 3), np.float32)
+        st = RenderStats()
+        check(self.lib.cgrt_render_views(self.h, arr, len(cams), C.byref(p), _vp(rgb), C.byref(st)))
+        return rgb, st.as_dict()
+
+    def render_views_device(self, cams, params, d_out_ptr, stream_ptr=0):
+        """Device form: [K][H][W][3] floats into d_out_ptr on the stream; statistics through collect_stats()."""
+        arr = (Camera * len(cams))(*cams)
+        check(self.lib.cgrt_render_views_device(self.h, arr, len(cams), C.byref(params), C.c_void_p(d_out_ptr),
+                                                C.c_void_p(stream_ptr)))
 
     def collect_stats(self):
         st = RenderStats()

@@ -7,6 +7,7 @@
 
 #include <algorithm>
 #include <cfloat>
+#include <climits>
 #include <cmath>
 #include <cstdio>
 #include <cstring>
@@ -1216,7 +1217,9 @@ static bool waveTuning(WaveQ& Q, int nSlots, int nLights, int world)
     return fin <= 0 && tune != 0;      // the finisher share may be tuned by measurement (WaveTuner)
 }
 
-static int prepareFrame(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render_params* p, FrameParams& P,
+// A frame of nViews cameras (cgrt_render_views) is one frame of nViews x the one-view pixel slots: the tile sequence and
+// primaryPixels stay those of one view, everything sized from P.nSlots grows with the views.
+static int prepareFrame(cgrt_scene* s, const cgrt_camera* cams, int nViews, const cgrt_render_params* p, FrameParams& P,
                         const int** dTileList, const int2** dTileSeq, FramePipeline* pipe)
 {
     const int tw = p->tile_w > 0 ? p->tile_w : 8, th = p->tile_h > 0 ? p->tile_h : 8;
@@ -1252,7 +1255,8 @@ static int prepareFrame(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render
     }
     const TileLayout& L = s->layout;
     std::memset(&P, 0, sizeof P);
-    cameraConstants(*cam, P);
+    cameraConstants(cams[0], P);
+    P.nViews = nViews;
     P.width = p->width;
     P.height = p->height;
     P.nLights = (int)s->lights.size();
@@ -1264,7 +1268,10 @@ static int prepareFrame(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render
     P.world = L.world;
     P.rank = p->rank;
     P.screenLayout = (L.world == 1 || (p->flags & CGRT_RENDER_SCREEN_LAYOUT)) ? 1 : 0;
-    P.nSlots = (int)L.lists[p->rank].size() * L.tileW * L.tileH;
+    // pixel slots count whole tiles: thin frames with large tiles have many more slots than pixels
+    const int64_t slots = (int64_t)nViews * (int64_t)L.lists[p->rank].size() * L.tileW * L.tileH;
+    if (slots > INT_MAX) return fail(CGRT_ERR_INVALID, "too many pixel slots: views x tiles x tile pixels must stay below 2^31");
+    P.nSlots = (int)slots;
     *dTileList = L.world > 1 ? s->tileList.p : nullptr;
     *dTileSeq = s->tileSeq.p;
     // queues sized for the worst case (every pixel hits, every hit bounces); only the used prefix is touched
@@ -1325,8 +1332,8 @@ static int prepareFrame(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render
     RC(s->pathPix.ensure(cap));
     RC(s->counts.ensure(CGRT_CNT_TOTAL * CGRT_MAX_CHAINS));
     RC(s->tests.ensure(6));
-    // parameter block: FrameParams header + lights (2 x float4 each)
-    const size_t need = CGRT_PARAM_BLOCK_HEADER + ((size_t)nL + (size_t)P.nSph) * 32;
+    // parameter block: FrameParams header + lights (2 x float4 each) + cameras (CGRT_VIEW_F4 x float4 each)
+    const size_t need = CGRT_PARAM_BLOCK_HEADER + ((size_t)nL + (size_t)P.nSph) * 32 + (size_t)nViews * CGRT_VIEW_F4 * 16;
     if (need > s->paramBlockBytes || !s->hParamRing) {
         CK(cudaDeviceSynchronize());
         if (s->hParamRing) cudaFreeHost(s->hParamRing);
@@ -1429,10 +1436,9 @@ static int waveQueues(cgrt_scene* s, cudaStream_t st, WaveQ& Q)
     return CGRT_OK;
 }
 
-int cgrt_render_device(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render_params* p, float* d_out, void* stream)
+// one frame of nViews cameras into d_out (cgrt_render_device: one camera; cgrt_render_views_device: several)
+static int renderDevice(cgrt_scene* s, const cgrt_camera* cams, int nViews, const cgrt_render_params* p, float* d_out, void* stream)
 {
-    if (!s || !cam || !d_out) return fail(CGRT_ERR_INVALID, "null argument");
-    RC(checkRenderParams(p));
     RC(useSceneDevice(s));
     std::lock_guard<std::mutex> lk(s->mu);
     cudaStream_t st = (cudaStream_t)stream;
@@ -1440,7 +1446,7 @@ int cgrt_render_device(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render_
     const int* dTiles = nullptr;
     const int2* dSeq = nullptr;
     FramePipeline pipe;
-    RC(prepareFrame(s, cam, p, P, &dTiles, &dSeq, &pipe));
+    RC(prepareFrame(s, cams, nViews, p, P, &dTiles, &dSeq, &pipe));
     if (P.screenLayout && P.world > 1 && pipe == PIPE_COUNT)
         return fail(CGRT_ERR_INVALID, "CGRT_RENDER_COUNT renders into the tile-major buffer; it cannot be combined with CGRT_RENDER_SCREEN_LAYOUT");
     // per-frame upload (camera constants + lights, read live from the scene like src/main.cpp:835-876 allows)
@@ -1458,7 +1464,15 @@ int cgrt_render_device(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render_
         hl[2 * (s->lights.size() + i)] = make_float4(q[0], q[1], q[2], q[3]);
         hl[2 * (s->lights.size() + i) + 1] = make_float4(q[4], q[5], q[6], 0.0f);
     }
-    const size_t bytes = CGRT_PARAM_BLOCK_HEADER + (s->lights.size() + (size_t)P.nSph) * 32;
+    float4* hc = hl + 2 * (s->lights.size() + (size_t)P.nSph); // the views' cameras follow the lights
+    for (int v = 0; v < nViews; v++) {
+        FrameParams C;
+        cameraConstants(cams[v], C);
+        hc[CGRT_VIEW_F4 * v] = make_float4(C.camX, C.camY, C.camZ, C.halfW);
+        hc[CGRT_VIEW_F4 * v + 1] = make_float4(C.qx, C.qy, C.qz, C.qw);
+        hc[CGRT_VIEW_F4 * v + 2] = make_float4(C.halfH, 0.0f, 0.0f, 0.0f);
+    }
+    const size_t bytes = CGRT_PARAM_BLOCK_HEADER + (s->lights.size() + (size_t)P.nSph) * 32 + (size_t)nViews * CGRT_VIEW_F4 * 16;
     CK(cudaMemcpyAsync(s->dParamBlock.p, slot, bytes, cudaMemcpyHostToDevice, st));
     const int maxKernels = CGRT_TRACE_MAX_KERNELS;
     if ((p->flags & CGRT_RENDER_PROFILE_ALL) && s->traceEvents.empty()) {
@@ -1522,6 +1536,36 @@ int cgrt_render_device(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render_
     return CGRT_OK;
 }
 
+int cgrt_render_device(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render_params* p, float* d_out, void* stream)
+{
+    if (!s || !cam || !d_out) return fail(CGRT_ERR_INVALID, "null argument");
+    RC(checkRenderParams(p));
+    return renderDevice(s, cam, 1, p, d_out, stream);
+}
+
+// the arguments cgrt_render_views refuses, checked before any CUDA call
+static int checkViews(const cgrt_scene* s, const cgrt_camera* cams, int32_t nViews, const cgrt_render_params* p, const float* out)
+{
+    if (!s || !cams || !out) return fail(CGRT_ERR_INVALID, "null argument");
+    RC(checkRenderParams(p));
+    if (nViews < 1 || nViews > CGRT_MAX_VIEWS) return fail(CGRT_ERR_INVALID, "n_views must be in 1..1024");
+    if ((int64_t)nViews * p->width * p->height > (int64_t)1 << 28) return fail(CGRT_ERR_INVALID, "views too large: n_views x width x height > 2^28");
+    if (p->world != 1) return fail(CGRT_ERR_INVALID, "cgrt_render_views renders whole frames (world == 1)");
+    if (p->flags & ~CGRT_RENDER_PROFILE_ALL) return fail(CGRT_ERR_INVALID, "cgrt_render_views takes the CGRT_RENDER_PROFILE_* flags only");
+    // pixel slots of whole tiles (tile size as makeTileLayout picks it; prepareFrame checks the same total for every frame)
+    const int64_t tw = p->tile_w > 0 ? p->tile_w : 8, th = p->tile_h > 0 ? p->tile_h : 8;
+    if (nViews * ((p->width + tw - 1) / tw) * tw * ((p->height + th - 1) / th) * th > INT_MAX)
+        return fail(CGRT_ERR_INVALID, "too many pixel slots: views x tiles x tile pixels must stay below 2^31");
+    return CGRT_OK;
+}
+
+int cgrt_render_views_device(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, const cgrt_render_params* p, float* d_out,
+                             void* stream)
+{
+    RC(checkViews(s, cams, n_views, p, d_out));
+    return renderDevice(s, cams, n_views, p, d_out, stream);
+}
+
 int cgrt_render_collect_stats(cgrt_scene* s, cgrt_render_stats* stats)
 {
     if (!s || !stats) return fail(CGRT_ERR_INVALID, "null argument");
@@ -1543,8 +1587,8 @@ int cgrt_render_collect_stats(cgrt_scene* s, cgrt_render_stats* stats)
         }
     }
     const FrameParams& P = s->lastParams;
-    // logical rays (SURVEY.md §8(d)): primary = pixels of this rank inside the image
-    const uint64_t primary = s->primaryPixels;
+    // logical rays (SURVEY.md §8(d)): primary = pixels of this rank inside the image, in every view
+    const uint64_t primary = s->primaryPixels * (uint64_t)P.nViews;
     stats->primary = primary;
     if (s->lastPipeline == PIPE_WAVE) { // persistent wavefront: the watchdog of k_wave (a warp waited for seconds) invalidates the frame
         int err = 0;
@@ -1723,6 +1767,25 @@ int cgrt_render(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render_params*
             }
         }
     }
+    if (stats) RC(cgrt_render_collect_stats(s, stats));
+    return CGRT_OK;
+}
+
+// ---- several views of one scene in one frame --------------------------------------------------------------------------------
+int cgrt_render_views(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, const cgrt_render_params* p, float* rgb,
+                      cgrt_render_stats* stats)
+{
+    RC(checkViews(s, cams, n_views, p, rgb));
+    RC(useSceneDevice(s));
+    std::lock_guard<std::mutex> hostLock(s->hostMu);
+    const size_t floats = (size_t)n_views * p->width * p->height * 3;
+    {
+        std::lock_guard<std::mutex> lk(s->mu);
+        RC(s->frame.ensure(floats));
+    }
+    RC(renderDevice(s, cams, n_views, p, s->frame.p, s->stream));
+    CK(cudaMemcpyAsync(rgb, s->frame.p, floats * sizeof(float), cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaStreamSynchronize(s->stream));
     if (stats) RC(cgrt_render_collect_stats(s, stats));
     return CGRT_OK;
 }

@@ -73,7 +73,7 @@ namespace cgrt {
                                           // layout): max of x + 1, row + 1, W - x, H - row; 0 = no pixel (counters start at zero)
 #define CGRT_CNT_TOTAL (CGRT_CNT_PATHS + 9)
 #define CGRT_MAX_PEERS 32                       // flags one signal launch can write (GPUs of one box)
-#define CGRT_PARAM_BLOCK_HEADER 128             // bytes reserved for FrameParams in the per-frame block; lights follow
+#define CGRT_PARAM_BLOCK_HEADER 128             // bytes reserved for FrameParams in the per-frame block; lights, then cameras follow
 
 // Per-frame constants, evaluated on the host with libm exactly as Trackball does (framework/src/trackball.cpp:70-73, 92-103)
 // so that device sinf/cosf/tanf never enter the picture. Uploaded once per render together with the lights.
@@ -89,7 +89,12 @@ struct FrameParams {
     int world, rank;
     int screenLayout;       // 1: pixels are written at their Screen position (row H-1-y); 0: tile-major buffer of this rank
     int nSph;               // spherical lights (2 x float4 each, after the point lights in the parameter block)
+    int nViews;             // cameras of the frame (cgrt_render_views; 1 otherwise). nSlots counts the slots of all views; the
+                            // views' camera constants follow the lights in the parameter block (CGRT_VIEW_F4 x float4 each)
 };
+// camera constants of one view in the parameter block: [camX camY camZ | halfW] [qx qy qz qw] [halfH | - - -]
+#define CGRT_VIEW_F4 3
+#define CGRT_MAX_VIEWS 1024
 
 // Four kernel sets render a frame; cgrt_capi.cu choosePipeline picks one per frame (all give the same pixels and ray counts):
 //   counting wavefront  CGRT_RENDER_COUNT                                         launchCountingFrame, CountBuffers

@@ -915,12 +915,14 @@ __global__ void __launch_bounds__(128, CGRT_WAVE_MINBLOCKS) k_wave(DevScene S, c
         for (int base = blockIdx.x * blockDim.x; base < n; base += gridDim.x * blockDim.x) {
             const int slot = base + threadIdx.x;
             bool push = false;
-            V3 o = mk3(P.camX, P.camY, P.camZ), d = mk3(0.0f, 0.0f, 0.0f);
+            V3 o = mk3(0.0f, 0.0f, 0.0f), d = mk3(0.0f, 0.0f, 0.0f);
             if (slot < n) {
-                int x, y, outIdx, local;
+                int x, y, outIdx, local, v;
                 B.pathDepth[slot] = 0;
-                if (seqToPixel(P, tileSeq, slot, x, y, outIdx, local)) {
-                    d = primaryDirection(P, x, y);
+                if (seqToPixel(P, tileSeq, slot, x, y, outIdx, local, v)) {
+                    const ViewCamera C = viewCamera(P, lights, v);
+                    o = C.o;
+                    d = primaryDirection(P, C, x, y);
                     bool enter = S.nSpheres > 0; // a ray that does not enter the tree (bvh.cpp:831-844) can only hit spheres
                     if (!enter && S.nNodes > 0) {
                         const float4 q0 = __ldg(S.nodes + 0), q1 = __ldg(S.nodes + 1);
