@@ -67,6 +67,11 @@ class RenderStats(C.Structure):
                     pipeline=int(self.pipeline))
 
 
+class AovBuffers(C.Structure):
+    """cgrt_aov_buffers: per-pixel buffers of cgrt_render_aovs (host or device pointers; None = not produced)."""
+    _fields_ = [("depth", C.c_void_p), ("tri", C.c_void_p), ("normal", C.c_void_p), ("hits", C.c_void_p)]
+
+
 EXPORTS = [
     "cgrt_version", "cgrt_last_error", "cgrt_device_count", "cgrt_scene_create", "cgrt_scene_destroy",
     "cgrt_scene_set_lights", "cgrt_scene_set_spheres", "cgrt_bvh_num_levels", "cgrt_bvh_num_nodes",
@@ -79,7 +84,7 @@ EXPORTS = [
     "cgrt_memset_device", "cgrt_memcpy_d2h_async", "cgrt_peer_export", "cgrt_peer_open", "cgrt_peer_close",
     "cgrt_flag_signal", "cgrt_flag_wait", "cgrt_bvh_fast_tree_stats", "cgrt_render_submit", "cgrt_render_wait",
     "cgrt_render_effects", "cgrt_scene_set_spherical_lights", "cgrt_debug_wave_timeline", "cgrt_debug_wave_tuner",
-    "cgrt_render_views", "cgrt_render_views_device",
+    "cgrt_render_views", "cgrt_render_views_device", "cgrt_render_aovs", "cgrt_render_aovs_device",
 ]
 
 _lib = None
@@ -129,6 +134,9 @@ def load_library(path=None):
         "cgrt_render_device": (C.c_int, [vp, C.POINTER(Camera), C.POINTER(RenderParams), vp, vp]),
         "cgrt_render_views": (C.c_int, [vp, C.POINTER(Camera), i32, C.POINTER(RenderParams), vp, C.POINTER(RenderStats)]),
         "cgrt_render_views_device": (C.c_int, [vp, C.POINTER(Camera), i32, C.POINTER(RenderParams), vp, vp]),
+        "cgrt_render_aovs": (C.c_int, [vp, C.POINTER(Camera), i32, C.POINTER(RenderParams), vp, C.POINTER(AovBuffers),
+                                        C.POINTER(RenderStats)]),
+        "cgrt_render_aovs_device": (C.c_int, [vp, C.POINTER(Camera), i32, C.POINTER(RenderParams), vp, C.POINTER(AovBuffers), vp]),
         "cgrt_render_collect_stats": (C.c_int, [vp, C.POINTER(RenderStats)]),
         "cgrt_tile_buffer_floats": (sz, [C.POINTER(RenderParams)]),
         "cgrt_tile_list": (C.c_int, [C.POINTER(RenderParams), i32, i32p, i32]),
@@ -370,6 +378,29 @@ class Scene:
         arr = (Camera * len(cams))(*cams)
         check(self.lib.cgrt_render_views_device(self.h, arr, len(cams), C.byref(params), C.c_void_p(d_out_ptr),
                                                 C.c_void_p(stream_ptr)))
+
+    def render_aovs(self, cams, W, H, trace_limit=2, tile=(0, 0), flags=0, depth=True, tri=True, normal=True, hits=True):
+        """cgrt_render_aovs: (rgb[K,H,W,3], {"depth": float32[K,H,W], "tri": int32[K,H,W], "normal": float32[K,H,W,3],
+        "hits": uint8[K,H,W]} with the requested keys only, stats dict summed over the views). Screen layout, like rgb."""
+        K = len(cams)
+        arr = (Camera * K)(*cams)
+        p = render_params(W, H, trace_limit, tile_w=tile[0], tile_h=tile[1], flags=flags)
+        rgb = np.zeros((K, H, W, 3), np.float32)
+        want = dict(depth=(depth, (K, H, W), np.float32), tri=(tri, (K, H, W), np.int32),
+                    normal=(normal, (K, H, W, 3), np.float32), hits=(hits, (K, H, W), np.uint8))
+        out = {k: np.zeros(shp, dt) for k, (on, shp, dt) in want.items() if on}
+        a = AovBuffers(*[out[k].ctypes.data if k in out else None for k in ("depth", "tri", "normal", "hits")])
+        st = RenderStats()
+        check(self.lib.cgrt_render_aovs(self.h, arr, K, C.byref(p), _vp(rgb), C.byref(a), C.byref(st)))
+        return rgb, out, st.as_dict()
+
+    def render_aovs_device(self, cams, params, d_rgb_ptr, d_aov_ptrs, stream_ptr=0):
+        """Device form: rgb [K][H][W][3] into d_rgb_ptr and the buffers of d_aov_ptrs (dict of device pointers with keys
+        depth / tri / normal / hits; a missing key or None = not produced) on the stream; statistics through collect_stats()."""
+        arr = (Camera * len(cams))(*cams)
+        a = AovBuffers(*[d_aov_ptrs.get(k) for k in ("depth", "tri", "normal", "hits")])
+        check(self.lib.cgrt_render_aovs_device(self.h, arr, len(cams), C.byref(params), C.c_void_p(d_rgb_ptr), C.byref(a),
+                                               C.c_void_p(stream_ptr)))
 
     def collect_stats(self):
         st = RenderStats()

@@ -291,6 +291,7 @@ struct cgrt_scene {
     DevBuf<int> pathPix, counts, tileList;
     DevBuf<unsigned long long> tests;
     DevBuf<float4> hitRec;
+    DevBuf<float> aovStage; // cgrt_render_aovs: the requested per-pixel buffers on the device before their copy to the host
     DevBuf<int> hitList, pathDepth, replayShadow;
     DevBuf<float4> replayQ;
     DevBuf<float4> cRay[2], cRes[2], sRay[2], sRes[2];
@@ -353,7 +354,7 @@ static void destroyScene(cgrt_scene* s)
     s->triN0.release(); s->triN1.release(); s->triN2.release(); s->mats.release(); s->spheres.release();
     s->origToLeaf.release(); s->refParent.release(); s->alwaysTri.release(); s->pairs.release(); s->wide.release(); s->dParamBlock.release(); s->hitQ.release(); s->bounceQ.release(); s->pathState.release();
     s->lit.release(); s->pathPix.release(); s->counts.release(); s->tileList.release(); s->tileSeq.release(); s->frame.release();
-    s->tests.release(); s->hitRec.release(); s->hitList.release(); s->pathDepth.release(); s->replayShadow.release(); s->replayQ.release();
+    s->tests.release(); s->hitRec.release(); s->aovStage.release(); s->hitList.release(); s->pathDepth.release(); s->replayShadow.release(); s->replayQ.release();
     for (int k = 0; k < 2; k++) { s->cRay[k].release(); s->cRes[k].release(); s->sRay[k].release(); s->sRes[k].release(); }
     s->softList.release(); s->soft.release();
     s->waveRays.release(); s->waveFin.release(); s->waveCtl.release(); s->waveTrace.release(); s->waveResume.release();
@@ -1436,8 +1437,10 @@ static int waveQueues(cgrt_scene* s, cudaStream_t st, WaveQ& Q)
     return CGRT_OK;
 }
 
-// one frame of nViews cameras into d_out (cgrt_render_device: one camera; cgrt_render_views_device: several)
-static int renderDevice(cgrt_scene* s, const cgrt_camera* cams, int nViews, const cgrt_render_params* p, float* d_out, void* stream)
+// one frame of nViews cameras into d_out (cgrt_render_device: one camera; cgrt_render_views_device: several); aov (optional,
+// whole frames of the path, round or wave pipeline only): the per-pixel buffers of cgrt_render_aovs
+static int renderDevice(cgrt_scene* s, const cgrt_camera* cams, int nViews, const cgrt_render_params* p, float* d_out, void* stream,
+                        const AovBuffers* aov = nullptr)
 {
     RC(useSceneDevice(s));
     std::lock_guard<std::mutex> lk(s->mu);
@@ -1525,6 +1528,11 @@ static int renderDevice(cgrt_scene* s, const cgrt_camera* cams, int nViews, cons
         break;
     }
     }
+    // the AOV pass reads the level-0 hit records the frame left (after the round pipeline's chains have joined on st); a black
+    // frame (trace limit 0) leaves no records and a stale pathDepth
+    if (aov)
+        launches += launchAovPass(s->dev, dP, P, s->hitRec.p, P.traceLimit > 0 ? s->pathDepth.p : nullptr, pipe == PIPE_PATHS,
+                                  s->pathPix.p, s->counts.p, dSeq, *aov, numSMs, st);
     s->lastPipeline = pipe;
     CK(cudaEventRecord(s->ev1, st));
     CK(cudaGetLastError());
@@ -1564,6 +1572,24 @@ int cgrt_render_views_device(cgrt_scene* s, const cgrt_camera* cams, int32_t n_v
 {
     RC(checkViews(s, cams, n_views, p, d_out));
     return renderDevice(s, cams, n_views, p, d_out, stream);
+}
+
+// the arguments cgrt_render_aovs refuses: those of cgrt_render_views, a null aov, and an aov that requests no buffer
+static int checkAovs(const cgrt_scene* s, const cgrt_camera* cams, int32_t nViews, const cgrt_render_params* p, const float* rgb,
+                     const cgrt_aov_buffers* aov)
+{
+    RC(checkViews(s, cams, nViews, p, rgb));
+    if (!aov) return fail(CGRT_ERR_INVALID, "null aov");
+    if (!aov->depth && !aov->tri && !aov->normal && !aov->hits) return fail(CGRT_ERR_INVALID, "cgrt_render_aovs: no buffer requested");
+    return CGRT_OK;
+}
+
+int cgrt_render_aovs_device(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, const cgrt_render_params* p, float* d_rgb,
+                            const cgrt_aov_buffers* d_aov, void* stream)
+{
+    RC(checkAovs(s, cams, n_views, p, d_rgb, d_aov));
+    const AovBuffers A = {d_aov->depth, d_aov->tri, d_aov->normal, d_aov->hits};
+    return renderDevice(s, cams, n_views, p, d_rgb, stream, &A);
 }
 
 int cgrt_render_collect_stats(cgrt_scene* s, cgrt_render_stats* stats)
@@ -1785,6 +1811,35 @@ int cgrt_render_views(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, c
     }
     RC(renderDevice(s, cams, n_views, p, s->frame.p, s->stream));
     CK(cudaMemcpyAsync(rgb, s->frame.p, floats * sizeof(float), cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaStreamSynchronize(s->stream));
+    if (stats) RC(cgrt_render_collect_stats(s, stats));
+    return CGRT_OK;
+}
+
+// ---- per-pixel buffers with the frame ------------------------------------------------------------------------------------------
+int cgrt_render_aovs(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, const cgrt_render_params* p, float* rgb,
+                     const cgrt_aov_buffers* aov, cgrt_render_stats* stats)
+{
+    RC(checkAovs(s, cams, n_views, p, rgb, aov));
+    RC(useSceneDevice(s));
+    std::lock_guard<std::mutex> hostLock(s->hostMu);
+    const size_t px = (size_t)n_views * p->width * p->height;
+    // staging on the device: depth [px] | tri [px] | normal [3 px] | hits [px bytes]
+    float* stage = nullptr;
+    {
+        std::lock_guard<std::mutex> lk(s->mu);
+        RC(s->frame.ensure(px * 3));
+        RC(s->aovStage.ensure(px * 5 + (px + 3) / 4));
+        stage = s->aovStage.p;
+    }
+    const AovBuffers A = {aov->depth ? stage : nullptr, aov->tri ? (int*)(stage + px) : nullptr,
+                          aov->normal ? stage + 2 * px : nullptr, aov->hits ? (uint8_t*)(stage + 5 * px) : nullptr};
+    RC(renderDevice(s, cams, n_views, p, s->frame.p, s->stream, &A));
+    CK(cudaMemcpyAsync(rgb, s->frame.p, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, s->stream));
+    if (aov->depth) CK(cudaMemcpyAsync(aov->depth, A.depth, px * sizeof(float), cudaMemcpyDeviceToHost, s->stream));
+    if (aov->tri) CK(cudaMemcpyAsync(aov->tri, A.tri, px * sizeof(int32_t), cudaMemcpyDeviceToHost, s->stream));
+    if (aov->normal) CK(cudaMemcpyAsync(aov->normal, A.normal, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, s->stream));
+    if (aov->hits) CK(cudaMemcpyAsync(aov->hits, A.hits, px, cudaMemcpyDeviceToHost, s->stream));
     CK(cudaStreamSynchronize(s->stream));
     if (stats) RC(cgrt_render_collect_stats(s, stats));
     return CGRT_OK;

@@ -773,8 +773,8 @@ struct PathsPolicy {
                 const int rec = path * B.levels + level;
                 float4* r = B.hitRec + 3 * (size_t)rec;
                 r[0] = make_float4(pointOn.x, pointOn.y, pointOn.z, i2f(mat));
-                r[1] = make_float4(nn.x, nn.y, nn.z, 0.0f);
-                r[2] = make_float4(rd.x, rd.y, rd.z, 0.0f);
+                r[1] = make_float4(nn.x, nn.y, nn.z, R.t);
+                r[2] = make_float4(rd.x, rd.y, rd.z, i2f(R.sphere >= 0 ? -2 - R.sphere : R.tri));
                 B.hitList[listPos] = rec;
                 B.pathDepth[path] = level + 1;
                 const float ksz = mat >= 0 ? __ldg(S.mats + 2 * mat + 1).z : 0.0f;
@@ -1632,8 +1632,8 @@ __global__ void __launch_bounds__(128) k_finish(DevScene S, const FrameParams* _
                 rec = slot * B.levels + level;
                 float4* h = B.hitRec + 3 * (size_t)rec;
                 h[0] = make_float4(pointOn.x, pointOn.y, pointOn.z, i2f(mat));
-                h[1] = make_float4(nn.x, nn.y, nn.z, 0.0f);
-                h[2] = make_float4(d.x, d.y, d.z, 0.0f);
+                h[1] = make_float4(nn.x, nn.y, nn.z, R.t);
+                h[2] = make_float4(d.x, d.y, d.z, i2f(R.sphere >= 0 ? -2 - R.sphere : R.tri));
                 B.pathDepth[slot] = level + 1;
                 const float ksz = mat >= 0 ? __ldg(S.mats + 2 * mat + 1).z : 0.0f;
                 bounce = !(ksz <= 0.01f) && level + 1 < P.traceLimit; // shade(): mirror test main.cpp:246, trace limit :267
@@ -1889,6 +1889,55 @@ __global__ void k_generate_rays(const FrameParams* __restrict__ Pp, float4* __re
     const V3 d = primaryDirection(P, x, y);
     rays[2 * (size_t)i] = make_float4(P.camX, P.camY, P.camZ, FLT_MAX);
     rays[2 * (size_t)i + 1] = make_float4(d.x, d.y, d.z, 0.0f);
+}
+
+// ---- per-pixel buffers (cgrt_render_aovs) from the level-0 hit records ---------------------------------------------------------
+// The primary rays of a frame are those of k_generate_rays and its level-0 records hold what writeHit reports for them, so the
+// buffers equal cgrt_intersect_closest on cgrt_generate_rays bit for bit. r == nullptr: the primary ray missed.
+RT_DEV void storeAov(const DevScene& S, const AovBuffers& A, int outIdx, int depth, const float4* __restrict__ r)
+{
+    float t = FLT_MAX;
+    int id = -1;
+    float4 n = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+    if (r) {
+        n = r[1];
+        t = n.w;
+        id = f2i(r[2].w);
+        if (id >= 0) id = f2i(__ldg(S.triV0 + id).w); // leaf order -> global id, as writeHit
+    }
+    if (A.depth) A.depth[outIdx] = t;
+    if (A.tri) A.tri[outIdx] = id;
+    if (A.normal) {
+        A.normal[3 * (size_t)outIdx] = n.x;
+        A.normal[3 * (size_t)outIdx + 1] = n.y;
+        A.normal[3 * (size_t)outIdx + 2] = n.z;
+    }
+    if (A.hits) A.hits[outIdx] = (uint8_t)depth;
+}
+
+// one thread per pixel slot (padding slots of edge tiles write nothing); pathDepth == nullptr: every pixel is a miss
+__global__ void __launch_bounds__(128) k_aov_slots(DevScene S, const FrameParams* __restrict__ Pp, const float4* __restrict__ hitRec,
+                                                   const int* __restrict__ pathDepth, const int2* __restrict__ tileSeq, AovBuffers A)
+{
+    const FrameParams P = *Pp;
+    const int levels = P.traceLimit > 1 ? P.traceLimit : 1;
+    for (int slot = blockIdx.x * blockDim.x + threadIdx.x; slot < P.nSlots; slot += gridDim.x * blockDim.x) {
+        int x, y, outIdx, local;
+        if (!seqToPixel(P, tileSeq, slot, x, y, outIdx, local)) continue;
+        const int depth = pathDepth ? pathDepth[slot] : 0;
+        storeAov(S, A, outIdx, depth, depth > 0 ? hitRec + 3 * (size_t)slot * levels : nullptr);
+    }
+}
+
+// path pipeline: one thread per path (primary rays that hit), after k_aov_slots has written every pixel as a miss
+__global__ void __launch_bounds__(128) k_aov_paths(DevScene S, const FrameParams* __restrict__ Pp, const float4* __restrict__ hitRec,
+                                                   const int* __restrict__ pathDepth, const int* __restrict__ pathPix,
+                                                   const int* __restrict__ counts, AovBuffers A)
+{
+    const int levels = Pp->traceLimit > 1 ? Pp->traceLimit : 1;
+    const int n = counts[CGRT_CNT_PATHS];
+    for (int path = blockIdx.x * blockDim.x + threadIdx.x; path < n; path += gridDim.x * blockDim.x)
+        storeAov(S, A, pathPix[path], pathDepth[path], hitRec + 3 * (size_t)path * levels);
 }
 
 // ---- synchronous host render, overlapped delivery: the bounding box of the pixels the shading pass coloured (counts[CGRT_CNT_BBOX],
@@ -2478,6 +2527,20 @@ int launchWavePipeline(const DevScene& S, const FrameParams* dP, const FramePara
     k_wave<<<grid, 128, 0, st>>>(S, hP, dLights, Q, B, dTileSeq, fb);
     traceEnd(tr, 2, st);
     return 1;
+}
+
+int launchAovPass(const DevScene& S, const FrameParams* dP, const FrameParams& hP, const float4* hitRec, const int* pathDepth,
+                  bool perPath, const int* pathPix, const int* counts, const int2* dTileSeq, const AovBuffers& A, int numSMs,
+                  cudaStream_t st)
+{
+    const int grid = gridFor((size_t)hP.nSlots, 128, numSMs * 16);
+    if (!perPath || !pathDepth) {
+        k_aov_slots<<<grid, 128, 0, st>>>(S, dP, hitRec, pathDepth, dTileSeq, A);
+        return 1;
+    }
+    k_aov_slots<<<grid, 128, 0, st>>>(S, dP, hitRec, nullptr, dTileSeq, A); // the misses have no record
+    k_aov_paths<<<grid, 128, 0, st>>>(S, dP, hitRec, pathDepth, pathPix, counts, A);
+    return 2;
 }
 
 void launchAssemble(const float* gathered, size_t perRankFloats, const int* tileLists, const int* tileCounts, int maxTiles,

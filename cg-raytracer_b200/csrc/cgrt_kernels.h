@@ -118,7 +118,7 @@ struct CountBuffers {
 // path from its primary ray through its mirror bounces and leaves one hit record per (path, level); all shadow rays of the
 // frame are then traced by one any-hit launch and one shading launch folds each path back to its pixel.
 struct PathBuffers {
-    float4* hitRec;    // [path * levels + level] 3 x float4: [P | matId] [N | -] [D | -]
+    float4* hitRec;    // [path * levels + level] 3 x float4: [P | matId] [N | t] [D | id] (hitRecordId)
     int* hitList;      // [i] = path * levels + level, compacted list of all hit records (shadow work items)
     uint8_t* lit;      // [(path * levels + level) * nLights + light] 1 = light reaches the point
     int* pathPix;      // [path] output index of the path's pixel
@@ -143,7 +143,7 @@ struct RoundBuffers {
     float4* cRes[2];
     float4* sRay[2];   // shadow rays, double-buffered by level parity
     float4* sRes[2];
-    float4* hitRec;    // [slot * levels + level] 3 x float4: [P | matId] [N | -] [D | -]
+    float4* hitRec;    // [slot * levels + level] 3 x float4: [P | matId] [N | t] [D | id] (hitRecordId)
     uint8_t* lit;      // [(slot * levels + level) * nLights + light]
     int* pathDepth;    // [slot] number of levels that recorded a hit (0: the pixel is already final)
     int* counts;
@@ -152,6 +152,16 @@ struct RoundBuffers {
     int* softList;     // hit records of the frame (slot * levels + level), compacted; softList[cap * levels] = their number
     float* soft;       // [(slot * levels + level) * nSph + light] fraction of the 200 sample rays that reach the light
     unsigned softSeed;
+};
+// hitRecordId: D.w of a hit record (bit-cast int) = the triangle's LEAF-ORDER index (global id: triV0[id].w), or -2 - s for
+// sphere s. N.w = t of the hit. The shading passes read neither lane; the AOV pass reads both from the level-0 records.
+
+// Per-pixel buffers of a frame (cgrt_render_aovs), Screen layout, view after view; a null pointer is not written.
+struct AovBuffers {
+    float* depth;   // t of the primary ray's closest hit, FLT_MAX on a miss
+    int* tri;       // global triangle id of that hit, -1 miss, -2 - s sphere s
+    float* normal;  // 3 floats: shading normal of that hit, 0 on a miss
+    uint8_t* hits;  // levels of the pixel's path that recorded a hit (pathDepth)
 };
 
 // ---- persistent wavefront (cgrt_wave.cuh): control block + ticket queue of the single-kernel frame ----------------------------
@@ -237,6 +247,12 @@ int waveGridBlocks(int numSMs); // co-resident CTAs of k_wave on this device (oc
 int launchWavePipeline(const DevScene& S, const FrameParams* dP, const FrameParams& hP, const float4* dLights,
                        const RoundBuffers& B, const WaveQ& Q, const int2* dTileSeq, float* fb, int numSMs, WaveTrace* tr,
                        cudaStream_t st);
+// The AOV pass after a frame of the path, round or wave pipeline (whole frames in Screen layout). pathDepth == nullptr: no
+// records (trace limit 0), every pixel is a miss; perPath: the path pipeline's records (per path, pathPix gives the pixel),
+// else one record chain per pixel slot. Returns the kernels it launched.
+int launchAovPass(const DevScene& S, const FrameParams* dP, const FrameParams& hP, const float4* hitRec, const int* pathDepth,
+                  bool perPath, const int* pathPix, const int* counts, const int2* dTileSeq, const AovBuffers& A, int numSMs,
+                  cudaStream_t st);
 void launchDeliverBox(const int* bbox, int W, int H, const float* frame, float* hostFrame, int numSMs, cudaStream_t st);
 void launchAssemble(const float* gathered, size_t perRankFloats, const int* tileLists, const int* tileCounts, int maxTiles,
                     int world, int tileW, int tileH, int tilesX, int width, int height, float* frame, int numSMs,

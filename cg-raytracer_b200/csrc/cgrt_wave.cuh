@@ -419,8 +419,8 @@ RT_DEV void waveFinishLoop(const DevScene& S, const FrameParams& P, const float4
                     rec = slot * B.levels + level;
                     float4* h = B.hitRec + 3 * (size_t)rec;
                     h[0] = make_float4(pointOn.x, pointOn.y, pointOn.z, i2f(mat));
-                    h[1] = make_float4(nn.x, nn.y, nn.z, 0.0f);
-                    h[2] = make_float4(d.x, d.y, d.z, 0.0f);
+                    h[1] = make_float4(nn.x, nn.y, nn.z, R.t);
+                    h[2] = make_float4(d.x, d.y, d.z, i2f(R.sphere >= 0 ? -2 - R.sphere : R.tri));
                     B.pathDepth[slot] = level + 1;
                     const float ksz = mat >= 0 ? __ldg(S.mats + 2 * mat + 1).z : 0.0f;
                     bounce = !(ksz <= 0.01f) && level + 1 < P.traceLimit; // shade(): mirror test main.cpp:246, trace limit :267

@@ -259,6 +259,32 @@ int cgrt_render_views(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, c
                       cgrt_render_stats* stats);
 int cgrt_render_views_device(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, const cgrt_render_params* p,
                              float* d_out, void* stream);
+/* Per-pixel buffers of a frame ("AOVs", a G-buffer): what each pixel's primary ray hit, for picking, depth-based passes and
+ * masks. Any pointer may be NULL: that buffer is not produced. */
+typedef struct cgrt_aov_buffers {
+    float* depth;   /* [n_views][H][W]    t of the primary ray's closest hit; the ray's t (FLT_MAX) on a miss */
+    int32_t* tri;   /* [n_views][H][W]    cgrt_hit.tri of that hit: global triangle id, -1 miss, -2 - s sphere s */
+    float* normal;  /* [n_views][H][W][3] cgrt_hit.normal of that hit (shading normal towards the ray); 0 on a miss */
+    uint8_t* hits;  /* [n_views][H][W]    trace() levels of the pixel's path that hit: 0 = primary miss, .. trace_limit */
+} cgrt_aov_buffers;
+/* cgrt_render_views with per-pixel buffers: the frame's renderer keeps the hit distance and the hit's id in its level-0 hit
+ * records, and one small pass after the frame writes the requested buffers from them (DESIGN.md 4.5).
+ *   Layout   every buffer is in Screen layout (row H-1-y), view after view, like rgb; n_views = 1 is a single frame.
+ *   Equality rgb is bit for bit what cgrt_render_views returns for the same arguments; so are the stats, except
+ *            kernel_launches, which also counts the AOV pass (device_ms covers it), and the reported pipeline is the same.
+ *            Per pixel, depth, tri and normal are bit for bit the t, tri and normal cgrt_intersect_closest returns for that
+ *            pixel's ray from cgrt_generate_rays(cams[v]).
+ *   Limit 0  the frame traces nothing: every pixel reports a miss and hits is 0.
+ *   Refused  (CGRT_ERR_INVALID, before any CUDA call): everything cgrt_render_views refuses (so whole frames only, no
+ *            CGRT_RENDER_COUNT, no CGRT_RENDER_SCREEN_LAYOUT), a null aov, an aov whose four pointers are all NULL.
+ * The host form copies rgb and each requested buffer back on the scene's stream and synchronises once. The _device form takes
+ * device pointers and is asynchronous on `stream`; its statistics come from cgrt_render_collect_stats.
+ * Measured on one B200 (1000 W power limit): the pass adds 0.018-0.024 ms to a 1080p frame (C3, trace limit 5: 1.072 vs
+ * 1.095 ms, DESIGN.md 4.5). */
+int cgrt_render_aovs(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, const cgrt_render_params* p, float* rgb,
+                     const cgrt_aov_buffers* aov, cgrt_render_stats* stats);
+int cgrt_render_aovs_device(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, const cgrt_render_params* p,
+                            float* d_rgb, const cgrt_aov_buffers* d_aov, void* stream);
 int cgrt_render_collect_stats(cgrt_scene* s, cgrt_render_stats* stats);
 /* renderRayTracing's optional passes around the path (UI toggles, default off, src/main.cpp:33-35):
  *   CGRT_EFFECT_ANTIALIAS   src/main.cpp:663-687: four rays per pixel = the pixel-corner rays of the (2W x 2H) frame, summed in
