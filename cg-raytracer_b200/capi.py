@@ -85,6 +85,7 @@ EXPORTS = [
     "cgrt_flag_signal", "cgrt_flag_wait", "cgrt_bvh_fast_tree_stats", "cgrt_render_submit", "cgrt_render_wait",
     "cgrt_render_effects", "cgrt_scene_set_spherical_lights", "cgrt_debug_wave_timeline", "cgrt_debug_wave_tuner",
     "cgrt_render_views", "cgrt_render_views_device", "cgrt_render_aovs", "cgrt_render_aovs_device",
+    "cgrt_render_effects_views", "cgrt_render_effects_views_device",
 ]
 
 _lib = None
@@ -160,6 +161,9 @@ def load_library(path=None):
         "cgrt_render_submit": (C.c_int, [vp, C.POINTER(Camera), C.POINTER(RenderParams), vp]),
         "cgrt_render_wait": (C.c_int, [vp]),
         "cgrt_render_effects": (C.c_int, [vp, C.POINTER(Camera), C.POINTER(RenderParams), i32, vp, C.POINTER(RenderStats)]),
+        "cgrt_render_effects_views": (C.c_int, [vp, C.POINTER(Camera), i32, C.POINTER(RenderParams), i32, vp,
+                                                 C.POINTER(RenderStats)]),
+        "cgrt_render_effects_views_device": (C.c_int, [vp, C.POINTER(Camera), i32, C.POINTER(RenderParams), i32, vp, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)  # AttributeError here = header/library drift
@@ -216,6 +220,14 @@ def class_names(stats):
     return [COUNT_CLASS_NAMES, KERNEL_CLASS_NAMES, ROUND_CLASS_NAMES, WAVE_CLASS_NAMES][stats["pipeline"]]
 RENDER_PROFILE_ALL, RENDER_COUNT, RENDER_SCREEN_LAYOUT = 0xF, 0x100, 0x200
 IPC_HANDLE_BYTES = 64
+
+
+EFFECT_ANTIALIAS, EFFECT_MOTION_BLUR, EFFECT_BLOOM = 1, 2, 4
+
+
+def effects_mask(antialias=False, motion_blur=False, bloom=False):
+    """The `effects` bits of cgrt_render_effects / cgrt_render_effects_views."""
+    return (EFFECT_ANTIALIAS if antialias else 0) | (EFFECT_MOTION_BLUR if motion_blur else 0) | (EFFECT_BLOOM if bloom else 0)
 
 
 def render_params(W, H, trace_limit=2, rank=0, world=1, tile_w=0, tile_h=0, flags=0):
@@ -353,6 +365,23 @@ class Scene:
         check(self.lib.cgrt_render_effects(self.h, C.byref(cam), C.byref(p), (1 if antialias else 0) | (2 if motion_blur else 0) | (4 if bloom else 0),
                                            _vp(rgb), C.byref(st)))
         return rgb, st.as_dict()
+
+    def render_effects_views(self, cams, W, H, trace_limit=2, antialias=False, motion_blur=False, bloom=False):
+        """cgrt_render_effects_views: the effects of render_effects for several cameras in one call: (rgb[K,H,W,3], stats dict
+        summed over the renders)."""
+        arr = (Camera * len(cams))(*cams)
+        p = render_params(W, H, trace_limit)
+        rgb = np.zeros((len(cams), H, W, 3), np.float32)
+        st = RenderStats()
+        check(self.lib.cgrt_render_effects_views(self.h, arr, len(cams), C.byref(p), effects_mask(antialias, motion_blur, bloom),
+                                                 _vp(rgb), C.byref(st)))
+        return rgb, st.as_dict()
+
+    def render_effects_views_device(self, cams, params, effects, d_out_ptr, stream_ptr=0):
+        """Device form: [K][H][W][3] floats into d_out_ptr on the stream; statistics through collect_stats()."""
+        arr = (Camera * len(cams))(*cams)
+        check(self.lib.cgrt_render_effects_views_device(self.h, arr, len(cams), C.byref(params), effects, C.c_void_p(d_out_ptr),
+                                                        C.c_void_p(stream_ptr)))
 
     def render_submit(self, cam, params, host_ptr):
         """Streaming form: enqueue one frame into page-locked host memory (see cgrt_render_submit)."""

@@ -283,6 +283,7 @@ struct cgrt_scene {
     unsigned char* hParamRing = nullptr; // RING x paramBlockBytes, pinned
     size_t paramBlockBytes = 0;
     int ringPos = 0;
+    cudaEvent_t ringCopied[RING] = {}; // recorded after each slot's copy: a slot is rewritten only once its copy has run
     DevBuf<unsigned char> dParamBlock;
 
     // wavefront queues
@@ -307,7 +308,15 @@ struct cgrt_scene {
     cudaEvent_t renderDone[2] = {nullptr, nullptr}, copyDone[2] = {nullptr, nullptr};
     DevBuf<float> streamFrame[2];
     DevBuf<float> fxA, fxB, fxC, fxM; // cgrt_render_effects: supersampled / shifted frame, accumulator, bloom output, bloom matrix
-    DevBuf<int> fxProg;               // bloom: finished columns per image row
+    DevBuf<int> fxProg;               // bloom: finished columns per image row, then the ticket counter
+    // cgrt_render_effects_views: the renders of the last call (host) and their counters, copied on the stream after each render:
+    // [render][FX_STATS_INTS] = counts of every chain | soft-shadow hit count | k_wave watchdog word
+    struct FxRender { FrameParams P; FramePipeline pipe; int chains; uint64_t primaryPixels; };
+    std::vector<FxRender> fxRenders;
+    DevBuf<int> fxStats;
+    uint64_t fxLaunches = 0;
+    bool fxLast = false;                       // the last call was an effects-views call: collect_stats sums fxRenders
+    cudaEvent_t fxEv[2] = {nullptr, nullptr}; // its first and last event
     bool slotUsed[2] = {false, false};
     uint64_t submitSeq = 0;
     int64_t fastStats[8] = {0, 0, 0, 0, 0, 0, 0, 0};
@@ -375,7 +384,9 @@ static void destroyScene(cgrt_scene* s)
     }
     s->streamFrame[0].release(); s->streamFrame[1].release();
     s->zeroFrame.release();
-    s->fxA.release(); s->fxB.release(); s->fxC.release(); s->fxM.release(); s->fxProg.release();
+    s->fxA.release(); s->fxB.release(); s->fxC.release(); s->fxM.release(); s->fxProg.release(); s->fxStats.release();
+    for (cudaEvent_t e : s->fxEv) if (e) cudaEventDestroy(e);
+    for (cudaEvent_t e : s->ringCopied) if (e) cudaEventDestroy(e);
     for (WaveTuner::Slot& sl : s->tuner.ring) { if (sl.a) cudaEventDestroy(sl.a); if (sl.b) cudaEventDestroy(sl.b); }
     if (s->ev0) cudaEventDestroy(s->ev0);
     if (s->ev1) cudaEventDestroy(s->ev1);
@@ -1453,6 +1464,10 @@ static int renderDevice(cgrt_scene* s, const cgrt_camera* cams, int nViews, cons
     if (P.screenLayout && P.world > 1 && pipe == PIPE_COUNT)
         return fail(CGRT_ERR_INVALID, "CGRT_RENDER_COUNT renders into the tile-major buffer; it cannot be combined with CGRT_RENDER_SCREEN_LAYOUT");
     // per-frame upload (camera constants + lights, read live from the scene like src/main.cpp:835-876 allows)
+    // the slot's previous frame may still be waiting for its copy (frames enqueued faster than the stream runs them)
+    cudaEvent_t& copied = s->ringCopied[s->ringPos];
+    if (copied) CK(cudaEventSynchronize(copied));
+    else CK(cudaEventCreateWithFlags(&copied, cudaEventDisableTiming));
     unsigned char* slot = s->hParamRing + (size_t)s->ringPos * s->paramBlockBytes;
     s->ringPos = (s->ringPos + 1) % cgrt_scene::RING;
     std::memcpy(slot, &P, sizeof P);
@@ -1477,6 +1492,7 @@ static int renderDevice(cgrt_scene* s, const cgrt_camera* cams, int nViews, cons
     }
     const size_t bytes = CGRT_PARAM_BLOCK_HEADER + (s->lights.size() + (size_t)P.nSph) * 32 + (size_t)nViews * CGRT_VIEW_F4 * 16;
     CK(cudaMemcpyAsync(s->dParamBlock.p, slot, bytes, cudaMemcpyHostToDevice, st));
+    CK(cudaEventRecord(copied, st));
     const int maxKernels = CGRT_TRACE_MAX_KERNELS;
     if ((p->flags & CGRT_RENDER_PROFILE_ALL) && s->traceEvents.empty()) {
         s->traceEvents.resize(2 * maxKernels);
@@ -1541,6 +1557,7 @@ static int renderDevice(cgrt_scene* s, const cgrt_camera* cams, int nViews, cons
     s->lastLaunches = (uint64_t)launches;
     s->lastParams = P;
     s->haveLast = true;
+    s->fxLast = false;
     return CGRT_OK;
 }
 
@@ -1592,51 +1609,26 @@ int cgrt_render_aovs_device(cgrt_scene* s, const cgrt_camera* cams, int32_t n_vi
     return renderDevice(s, cams, n_views, p, d_rgb, stream, &A);
 }
 
-int cgrt_render_collect_stats(cgrt_scene* s, cgrt_render_stats* stats)
+// One frame's ray statistics (primary, primary_hit, shadow, bounce, replayed_*, pipeline) into a zeroed *stats: counts = its counters
+// summed over its chains, softHits = its records with soft-shadow samples (read only with spherical lights on a pipeline with
+// slot records), primaryPixels = the pixels of one view.
+static void frameRayStats(const FrameParams& P, FramePipeline pipe, const int* counts, int softHits, uint64_t primaryPixels,
+                          cgrt_render_stats* stats)
 {
-    if (!s || !stats) return fail(CGRT_ERR_INVALID, "null argument");
-    RC(useSceneDevice(s));
-    std::lock_guard<std::mutex> lk(s->mu);
-    std::memset(stats, 0, sizeof *stats);
-    if (!s->haveLast) return fail(CGRT_ERR_INVALID, "no frame rendered yet");
-    CK(cudaStreamSynchronize(s->lastStream));
-    int counts[CGRT_CNT_TOTAL];
-    const bool onHost = s->statsOnHost && s->hStats != nullptr;
-    {
-        const int nc = chainsOf(s);
-        std::vector<int> all((size_t)CGRT_CNT_TOTAL * nc);
-        if (onHost) std::memcpy(all.data(), s->hStats, all.size() * sizeof(int));
-        else CK(cudaMemcpy(all.data(), s->counts.p, all.size() * sizeof(int), cudaMemcpyDeviceToHost));
-        for (int k = 0; k < CGRT_CNT_TOTAL; k++) {
-            counts[k] = 0;
-            for (int c = 0; c < nc; c++) counts[k] += all[(size_t)c * CGRT_CNT_TOTAL + k];
-        }
-    }
-    const FrameParams& P = s->lastParams;
     // logical rays (SURVEY.md §8(d)): primary = pixels of this rank inside the image, in every view
-    const uint64_t primary = s->primaryPixels * (uint64_t)P.nViews;
-    stats->primary = primary;
-    if (s->lastPipeline == PIPE_WAVE) { // persistent wavefront: the watchdog of k_wave (a warp waited for seconds) invalidates the frame
-        int err = 0;
-        if (onHost) err = s->hStats[CGRT_CNT_TOTAL * CGRT_MAX_CHAINS];
-        else CK(cudaMemcpy(&err, s->waveCtl.p + WCTL_ERR, sizeof(int), cudaMemcpyDeviceToHost));
-        if (err) return fail(CGRT_ERR_CUDA, "k_wave watchdog: the persistent wavefront did not complete; the frame is invalid");
-    }
-    stats->pipeline = s->lastPipeline;
-    if (hasSlotRecords(s->lastPipeline)) {
+    stats->primary = primaryPixels * (uint64_t)P.nViews;
+    stats->pipeline = pipe;
+    if (hasSlotRecords(pipe)) {
         stats->primary_hit = (uint64_t)counts[CGRT_CNT_PATHS];
         for (int l = 0; l < P.traceLimit; l++) {
             stats->shadow += (uint64_t)counts[CGRT_CNT_HIT + l] * (uint64_t)P.nLights;
             if (l >= 1) stats->bounce += (uint64_t)counts[CGRT_CNT_BOUNCE + l];
         }
-        if (P.nSph > 0) { // 200 sample rays per hit record and spherical light (main.cpp:177)
-            int nHits = 0;
-            CK(cudaMemcpy(&nHits, s->softList.p + (size_t)std::max(P.nSlots, 1) * std::max(P.traceLimit, 1), sizeof(int), cudaMemcpyDeviceToHost));
-            stats->shadow += 200ull * (uint64_t)nHits * (uint64_t)P.nSph;
-        }
+        if (P.nSph > 0) // 200 sample rays per hit record and spherical light (main.cpp:177)
+            stats->shadow += 200ull * (uint64_t)softHits * (uint64_t)P.nSph;
         stats->replayed_closest = (uint32_t)counts[CGRT_CNT_REPLAY_PATHS];
         stats->replayed_shadow = (uint32_t)counts[CGRT_CNT_REPLAY_SHADOW];
-    } else if (s->lastPipeline == PIPE_PATHS) {
+    } else if (pipe == PIPE_PATHS) {
         stats->primary_hit = (uint64_t)counts[CGRT_CNT_PATHS];
         stats->shadow = (uint64_t)counts[CGRT_CNT_HITS] * (uint64_t)P.nLights;
         stats->bounce = (uint64_t)counts[CGRT_CNT_BOUNCES];
@@ -1650,6 +1642,79 @@ int cgrt_render_collect_stats(cgrt_scene* s, cgrt_render_stats* stats)
         }
     }
     if (P.traceLimit == 0) stats->primary = 0;
+}
+// where the soft-shadow hit count of a frame sits (after its hit-record list)
+static const int* softHitCount(const cgrt_scene* s, const FrameParams& P)
+{
+    return s->softList.p + (size_t)std::max(P.nSlots, 1) * std::max(P.traceLimit, 1);
+}
+// ints per render of an effects-views call in fxStats: the counters of every chain, the soft-shadow hit count, the watchdog word
+static const int FX_STATS_INTS = CGRT_CNT_TOTAL * CGRT_MAX_CHAINS + 2;
+
+// the statistics of an effects-views call: each render's by frameRayStats, summed (after the stream has synchronised)
+static int collectEffectsStats(cgrt_scene* s, cgrt_render_stats* stats)
+{
+    std::vector<int> all(s->fxRenders.size() * FX_STATS_INTS);
+    CK(cudaMemcpy(all.data(), s->fxStats.p, all.size() * sizeof(int), cudaMemcpyDeviceToHost));
+    for (size_t r = 0; r < s->fxRenders.size(); r++) {
+        const cgrt_scene::FxRender& R = s->fxRenders[r];
+        const int* c = all.data() + r * FX_STATS_INTS;
+        if (R.pipe == PIPE_WAVE && c[FX_STATS_INTS - 1])
+            return fail(CGRT_ERR_CUDA, "k_wave watchdog: the persistent wavefront did not complete; the frame is invalid");
+        int counts[CGRT_CNT_TOTAL];
+        for (int k = 0; k < CGRT_CNT_TOTAL; k++) {
+            counts[k] = 0;
+            for (int ch = 0; ch < R.chains; ch++) counts[k] += c[ch * CGRT_CNT_TOTAL + k];
+        }
+        cgrt_render_stats one;
+        std::memset(&one, 0, sizeof one);
+        frameRayStats(R.P, R.pipe, counts, c[CGRT_CNT_TOTAL * CGRT_MAX_CHAINS], R.primaryPixels, &one);
+        stats->primary += one.primary;
+        stats->primary_hit += one.primary_hit;
+        stats->shadow += one.shadow;
+        stats->bounce += one.bounce;
+        stats->replayed_closest += one.replayed_closest;
+        stats->replayed_shadow += one.replayed_shadow;
+        stats->pipeline = one.pipeline;
+    }
+    stats->kernel_launches = s->fxLaunches;
+    float ms = 0.0f;
+    CK(cudaEventElapsedTime(&ms, s->fxEv[0], s->fxEv[1]));
+    stats->device_ms = ms;
+    return CGRT_OK;
+}
+
+int cgrt_render_collect_stats(cgrt_scene* s, cgrt_render_stats* stats)
+{
+    if (!s || !stats) return fail(CGRT_ERR_INVALID, "null argument");
+    RC(useSceneDevice(s));
+    std::lock_guard<std::mutex> lk(s->mu);
+    std::memset(stats, 0, sizeof *stats);
+    if (!s->haveLast) return fail(CGRT_ERR_INVALID, "no frame rendered yet");
+    CK(cudaStreamSynchronize(s->lastStream));
+    if (s->fxLast) return collectEffectsStats(s, stats);
+    int counts[CGRT_CNT_TOTAL];
+    const bool onHost = s->statsOnHost && s->hStats != nullptr;
+    {
+        const int nc = chainsOf(s);
+        std::vector<int> all((size_t)CGRT_CNT_TOTAL * nc);
+        if (onHost) std::memcpy(all.data(), s->hStats, all.size() * sizeof(int));
+        else CK(cudaMemcpy(all.data(), s->counts.p, all.size() * sizeof(int), cudaMemcpyDeviceToHost));
+        for (int k = 0; k < CGRT_CNT_TOTAL; k++) {
+            counts[k] = 0;
+            for (int c = 0; c < nc; c++) counts[k] += all[(size_t)c * CGRT_CNT_TOTAL + k];
+        }
+    }
+    const FrameParams& P = s->lastParams;
+    if (s->lastPipeline == PIPE_WAVE) { // persistent wavefront: the watchdog of k_wave (a warp waited for seconds) invalidates the frame
+        int err = 0;
+        if (onHost) err = s->hStats[CGRT_CNT_TOTAL * CGRT_MAX_CHAINS];
+        else CK(cudaMemcpy(&err, s->waveCtl.p + WCTL_ERR, sizeof(int), cudaMemcpyDeviceToHost));
+        if (err) return fail(CGRT_ERR_CUDA, "k_wave watchdog: the persistent wavefront did not complete; the frame is invalid");
+    }
+    int softHits = 0;
+    if (hasSlotRecords(s->lastPipeline) && P.nSph > 0) CK(cudaMemcpy(&softHits, softHitCount(s, P), sizeof(int), cudaMemcpyDeviceToHost));
+    frameRayStats(P, s->lastPipeline, counts, softHits, s->primaryPixels, stats);
     stats->kernel_launches = s->lastLaunches;
     float ms = 0.0f;
     CK(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
@@ -1876,9 +1941,9 @@ int cgrt_render_effects(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render
         RC(s->fxA.ensure(n));
         RC(s->fxC.ensure(n));
         RC(s->fxM.ensure(n));
-        RC(s->fxProg.ensure((size_t)H));
+        RC(s->fxProg.ensure((size_t)H + 1));
         RC(cgrt_render_device(s, cam, p, s->fxA.p, st));
-        launchBloom(s->fxA.p, W, H, s->fxM.p, s->fxProg.p, s->fxC.p, s->di.numSMs, st);
+        launchBloom(s->fxA.p, W, H, 1, s->fxM.p, s->fxProg.p, s->fxC.p, s->di.numSMs, st);
         CK(cudaGetLastError());
         if (stats) {
             cgrt_render_stats one;
@@ -1930,7 +1995,7 @@ int cgrt_render_effects(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render
         RC(s->fxA.ensure(n * 4));
         RC(s->fxB.ensure(n));
         RC(cgrt_render_device(s, cam, &big, s->fxA.p, st)); // aspect stays cam->aspect (W/H)
-        launchAADownsample(s->fxA.p, W, H, s->fxB.p, st);
+        launchAADownsample(s->fxA.p, W, H, 1, s->fxB.p, st);
         CK(cudaGetLastError());
         CK(cudaMemcpyAsync(rgb, s->fxB.p, n * sizeof(float), cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
@@ -1942,6 +2007,155 @@ int cgrt_render_effects(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render
         }
     }
     if (stats) *stats = total;
+    return CGRT_OK;
+}
+
+// ---- the effects for several views, on the caller's stream ----------------------------------------------------------------
+// Pixel slots of one render of an effects-views call: the cameras of a render share it up to this many slots (about the 15
+// motion-blur cameras of a 1080p view); a render of one camera may be larger.
+static const int64_t FX_BATCH_SLOTS = (int64_t)1 << 25;
+
+// the arguments cgrt_render_effects_views refuses, checked before any CUDA call (the bloom height check needs the device)
+static int checkEffectsViews(const cgrt_scene* s, const cgrt_camera* cams, int32_t nViews, const cgrt_render_params* p,
+                             int32_t effects, const float* out)
+{
+    if (!s || !cams || !out) return fail(CGRT_ERR_INVALID, "null argument");
+    RC(checkRenderParams(p));
+    if (nViews < 1 || nViews > CGRT_MAX_VIEWS) return fail(CGRT_ERR_INVALID, "n_views must be in 1..1024");
+    if ((int64_t)nViews * p->width * p->height > (int64_t)1 << 28) return fail(CGRT_ERR_INVALID, "views too large: n_views x width x height > 2^28");
+    if (p->world != 1) return fail(CGRT_ERR_INVALID, "cgrt_render_effects_views renders whole frames (world == 1)");
+    if (p->flags != 0) return fail(CGRT_ERR_INVALID, "cgrt_render_effects_views takes no render flags");
+    if (effects & ~(CGRT_EFFECT_ANTIALIAS | CGRT_EFFECT_MOTION_BLUR | CGRT_EFFECT_BLOOM)) return fail(CGRT_ERR_INVALID, "unknown effect bits");
+    if ((effects & CGRT_EFFECT_BLOOM) && (effects & CGRT_EFFECT_ANTIALIAS))
+        return fail(CGRT_ERR_INVALID, "bloom with anti-aliasing is not offered (see cgrt_render_effects)");
+    if (effects == CGRT_EFFECT_ANTIALIAS && (int64_t)p->width * 2 * p->height * 2 > (int64_t)1 << 28)
+        return fail(CGRT_ERR_INVALID, "frame too large for 2x2 supersampling");
+    return CGRT_OK;
+}
+
+// Cameras [c0, c1) of a list of nViews x perView cameras, per render: as many whole views as FX_BATCH_SLOTS allows, or, when one
+// view's cameras do not fit, that view's cameras in order over several renders.
+static std::vector<std::pair<int, int>> fxBatches(int nViews, int perView, const cgrt_render_params& p)
+{
+    const int64_t tw = p.tile_w > 0 ? p.tile_w : 8, th = p.tile_h > 0 ? p.tile_h : 8;
+    const int64_t slots = (p.width + tw - 1) / tw * tw * ((p.height + th - 1) / th * th);
+    const int64_t fit = std::max<int64_t>(1, FX_BATCH_SLOTS / slots);
+    const int total = nViews * perView;
+    std::vector<std::pair<int, int>> b;
+    if (fit >= perView) {
+        const int step = (int)std::min<int64_t>(fit / perView, nViews) * perView;
+        for (int c = 0; c < total; c += step) b.push_back(std::make_pair(c, std::min(c + step, total)));
+    } else {
+        for (int v = 0; v < nViews; v++)
+            for (int k = 0; k < perView; k += (int)fit) b.push_back(std::make_pair(v * perView + k, v * perView + std::min(k + (int)fit, perView)));
+    }
+    return b;
+}
+
+// one render of an effects-views call: the frame, then its counters copied on the stream into the call's next fxStats entry
+static int fxRender(cgrt_scene* s, const cgrt_camera* cams, int n, const cgrt_render_params* p, float* d_out, cudaStream_t st)
+{
+    RC(renderDevice(s, cams, n, p, d_out, st));
+    std::lock_guard<std::mutex> lk(s->mu);
+    const cgrt_scene::FxRender R = {s->lastParams, s->lastPipeline, chainsOf(s), s->primaryPixels};
+    int* dst = s->fxStats.p + s->fxRenders.size() * FX_STATS_INTS;
+    CK(cudaMemcpyAsync(dst, s->counts.p, sizeof(int) * CGRT_CNT_TOTAL * R.chains, cudaMemcpyDeviceToDevice, st));
+    if (hasSlotRecords(R.pipe) && R.P.nSph > 0)
+        CK(cudaMemcpyAsync(dst + CGRT_CNT_TOTAL * CGRT_MAX_CHAINS, softHitCount(s, R.P), sizeof(int), cudaMemcpyDeviceToDevice, st));
+    if (R.pipe == PIPE_WAVE) CK(cudaMemcpyAsync(dst + FX_STATS_INTS - 1, s->waveCtl.p + WCTL_ERR, sizeof(int), cudaMemcpyDeviceToDevice, st));
+    s->fxRenders.push_back(R);
+    s->fxLaunches += s->lastLaunches;
+    return CGRT_OK;
+}
+
+int cgrt_render_effects_views_device(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, const cgrt_render_params* p,
+                                     int32_t effects, float* d_out, void* stream)
+{
+    RC(checkEffectsViews(s, cams, n_views, p, effects, d_out));
+    if (!effects) return cgrt_render_views_device(s, cams, n_views, p, d_out, stream);
+    RC(useSceneDevice(s));
+    cudaStream_t st = (cudaStream_t)stream;
+    const int W = p->width, H = p->height, V = n_views;
+    const size_t n = (size_t)W * H * 3; // floats of one view
+    const bool blur = (effects & CGRT_EFFECT_MOTION_BLUR) != 0, bloom = (effects & CGRT_EFFECT_BLOOM) != 0;
+    if (bloom && (int64_t)H > (int64_t)s->di.numSMs * 16 * 4) return fail(CGRT_ERR_INVALID, "frame too tall for the bloom pass");
+    // the renders: the un-shifted views (bloom), the 15 shifted cameras of every view (motion blur) or the 2W x 2H views
+    cgrt_render_params big = *p;
+    std::vector<cgrt_camera> shifted;
+    if (blur) {
+        static const double shift[15] = {0.01, 0.02, 0.03, 0.04, 0.05, 0.06, 0.07, 0.08, 0.09, 0.10, 0.11, 0.12, 0.13, 0.14, 0.15};
+        shifted.resize((size_t)V * 15);
+        for (int v = 0; v < V; v++)
+            for (int k = 0; k < 15; k++) { // cameraNew.setLookAt(glm::vec3(0.0k, 0, 0)), main.cpp:344-568
+                cgrt_camera& c = shifted[(size_t)v * 15 + k];
+                c = cams[v];
+                c.look_at[0] = (float)shift[k];
+                c.look_at[1] = 0.0f;
+                c.look_at[2] = 0.0f;
+            }
+    } else if (!bloom) {
+        big.width = 2 * W;
+        big.height = 2 * H;
+    }
+    const std::vector<std::pair<int, int>> plain = bloom ? fxBatches(V, 1, *p) : std::vector<std::pair<int, int>>();
+    const std::vector<std::pair<int, int>> batches = blur ? fxBatches(V, 15, *p) : (bloom ? std::vector<std::pair<int, int>>() : fxBatches(V, 1, big));
+    size_t batchFrames = 0;
+    for (const auto& b : batches) batchFrames = std::max(batchFrames, (size_t)(b.second - b.first));
+    {
+        std::lock_guard<std::mutex> lk(s->mu);
+        RC(s->fxStats.ensure((plain.size() + batches.size()) * FX_STATS_INTS));
+        RC(s->fxA.ensure(batchFrames * n * (blur ? 1 : 4)));
+        if (bloom) {
+            RC(s->fxB.ensure((size_t)V * n));
+            RC(s->fxM.ensure((size_t)V * n));
+            RC(s->fxProg.ensure((size_t)V * H + 1));
+        }
+        for (cudaEvent_t& e : s->fxEv)
+            if (!e) CK(cudaEventCreate(&e));
+        s->fxRenders.clear();
+        s->fxLaunches = 0;
+        CK(cudaEventRecord(s->fxEv[0], st));
+    }
+    int launches = 0;
+    if (bloom) { // bloomEffect (main.cpp:698-705, 586-628) of every view in one pass; its output goes straight to d_out
+        for (const auto& b : plain) RC(fxRender(s, cams + b.first, b.second - b.first, p, s->fxB.p + (size_t)b.first * n, st));
+        launchBloom(s->fxB.p, W, H, V, s->fxM.p, s->fxProg.p, d_out, s->di.numSMs, st);
+        launches += 2;
+    }
+    for (const auto& b : batches) {
+        if (blur) { // blurEffect (main.cpp:716-719, :581): overwrites every pixel, whatever the loop drew
+            RC(fxRender(s, shifted.data() + b.first, b.second - b.first, p, s->fxA.p, st));
+            launchBlurViews(s->fxA.p, b.first, b.second, n, bloom ? s->fxB.p : nullptr, d_out, 16.0f, st);
+        } else { // anti-aliasing; the aspect stays cams[v].aspect (W/H)
+            RC(fxRender(s, cams + b.first, b.second - b.first, &big, s->fxA.p, st));
+            launchAADownsample(s->fxA.p, W, H, b.second - b.first, d_out + (size_t)b.first * n, st);
+        }
+        launches++;
+    }
+    CK(cudaGetLastError());
+    std::lock_guard<std::mutex> lk(s->mu);
+    CK(cudaEventRecord(s->fxEv[1], st));
+    s->fxLaunches += (uint64_t)launches;
+    s->fxLast = true;
+    return CGRT_OK;
+}
+
+int cgrt_render_effects_views(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, const cgrt_render_params* p, int32_t effects,
+                              float* rgb, cgrt_render_stats* stats)
+{
+    RC(checkEffectsViews(s, cams, n_views, p, effects, rgb));
+    if (!effects) return cgrt_render_views(s, cams, n_views, p, rgb, stats);
+    RC(useSceneDevice(s));
+    std::lock_guard<std::mutex> hostLock(s->hostMu);
+    const size_t floats = (size_t)n_views * p->width * p->height * 3;
+    {
+        std::lock_guard<std::mutex> lk(s->mu);
+        RC(s->frame.ensure(floats));
+    }
+    RC(cgrt_render_effects_views_device(s, cams, n_views, p, effects, s->frame.p, s->stream));
+    CK(cudaMemcpyAsync(rgb, s->frame.p, floats * sizeof(float), cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaStreamSynchronize(s->stream));
+    if (stats) RC(cgrt_render_collect_stats(s, stats));
     return CGRT_OK;
 }
 

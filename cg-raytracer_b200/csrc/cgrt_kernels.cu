@@ -2017,10 +2017,14 @@ __global__ void k_quantize(const float* __restrict__ frame, size_t nPixels, uint
 // level = 2, i.e. exactly the pixel-corner rays of a (2W x 2H) frame (float(k)/(2W)*2 == float(k)/W*1 bit for bit), summed in
 // the order (j outer, i inner) into `color` and divided by level * 2.5 = 5 (sic). `color` is never initialised in the reference;
 // this implementation starts it at zero (documented assumption).
-__global__ void k_aa_downsample(const float* __restrict__ big, int W, int H, float* __restrict__ out)
+__global__ void k_aa_downsample(const float* __restrict__ big, int W, int H, int nViews, float* __restrict__ out)
 {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= W * H) return;
+    const size_t px = (size_t)W * H;
+    const size_t iv = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (iv >= px * nViews) return;
+    const size_t v = iv / px;
+    const int i = (int)(iv - v * px);
+    big += v * px * 12; // one view's 2W x 2H x 3 floats
     const int row = i / W, x = i - row * W; // Screen layout: row = H-1-y
     const int y = H - 1 - row;
     const int W2 = 2 * W, H2 = 2 * H;
@@ -2033,9 +2037,9 @@ __global__ void k_aa_downsample(const float* __restrict__ big, int W, int H, flo
         }
     const float level = 2.0f;
     const float div = level * 2.5f;
-    out[3 * (size_t)i + 0] = c[0] / div;
-    out[3 * (size_t)i + 1] = c[1] / div;
-    out[3 * (size_t)i + 2] = c[2] / div;
+    out[3 * iv + 0] = c[0] / div;
+    out[3 * iv + 1] = c[1] / div;
+    out[3 * iv + 2] = c[2] / div;
 }
 
 // Motion blur (blurEffect, main.cpp:318-584): matrixPixels += frame for the 15 shifted look-at points, then / 16
@@ -2051,6 +2055,27 @@ __global__ void k_divide(const float* __restrict__ acc, size_t n, float div, flo
     if (i >= n) return;
     out[i] = acc[i] / div;
 }
+// Motion blur of several views (cgrt_render_effects_views): `frames` holds the cameras c0..c1-1 of the flattened list c = 15 v + k
+// (k = 0..14 <-> look-at (0.01 (k + 1), 0, 0)), one W x H x 3 block each; this adds each view's cameras into its entry of acc in
+// the order of k - the running sum k_accumulate builds one frame at a time: 0 + f_0 (without bloom) or (0 + A) + C (with bloom:
+// A the un-shifted frame in bloomIn, C its bloom output, which acc holds) + f_0, then + f_k - and divides by div after k = 14.
+// A view's cameras may be spread over several launches; they come in order of k.
+__global__ void k_blur_views(const float* __restrict__ frames, int c0, int c1, size_t n, const float* __restrict__ bloomIn,
+                             float* __restrict__ acc, float div)
+{
+    const int v0 = c0 / 15;
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const size_t vl = i / n;
+    if (vl >= (size_t)((c1 - 1) / 15 - v0 + 1)) return;
+    const int v = v0 + (int)vl;
+    const size_t e = i - vl * n, o = (size_t)v * n + e;
+    const int ka = max(c0, 15 * v) - 15 * v, kb = min(c1, 15 * v + 15) - 15 * v; // this view's cameras in the launch
+    float a;
+    if (ka == 0) a = bloomIn ? (0.0f + bloomIn[o]) + acc[o] : 0.0f;
+    else a = acc[o];
+    for (int k = ka; k < kb; k++) a = a + frames[(size_t)(15 * v + k - c0) * n + e];
+    acc[o] = kb == 15 ? a / div : a;
+}
 
 // ---- bloom (bloomEffect, src/main.cpp:586-628; bookkeeping :698-705) --------------------------------------------------------------
 // The reference keeps the pixels whose colour sums to more than 1 (matrixColorsScreen, else black) and then replaces every entry,
@@ -2062,29 +2087,45 @@ __global__ void k_divide(const float* __restrict__ acc, size_t n, float div, flo
 // row, rows chasing each other 11 columns apart (~W / 11 rows in flight), each warp keeping its 21 x 21 window in shared memory
 // (one new column per step) and adding the up to 440 terms of an entry in the reference's order - the additions of one entry
 // are a dependent chain by definition (float addition is not associative), the three channels are three lanes.
-// k_bloom_init: M[y * W + x] = thresholded colour in the reference's index order (ray space: image row H - 1 - y), progress = 0.
-__global__ void k_bloom_init(const float* __restrict__ frame, int W, int H, float* __restrict__ M, int* __restrict__ progress)
+// k_bloom_init: M[y * W + x] = thresholded colour in the reference's index order (ray space: image row H - 1 - y), progress = 0,
+// for each of nViews frames; progress[nViews * H] is the ticket counter of k_bloom.
+__global__ void k_bloom_init(const float* __restrict__ frame, int W, int H, int nViews, float* __restrict__ M, int* __restrict__ progress)
 {
-    const size_t n = (size_t)W * H;
+    const size_t px = (size_t)W * H, n = px * nViews;
     for (size_t p = blockIdx.x * (size_t)blockDim.x + threadIdx.x; p < n; p += (size_t)gridDim.x * blockDim.x) {
-        const int y = (int)(p / W), x = (int)(p - (size_t)y * W);
-        const float* c = frame + 3 * ((size_t)(H - 1 - y) * W + x);
+        const size_t v = p / px;
+        const size_t q = p - v * px;
+        const int y = (int)(q / W), x = (int)(q - (size_t)y * W);
+        const float* c = frame + 3 * (v * px + (size_t)(H - 1 - y) * W + x);
         const bool keep = c[0] + c[1] + c[2] > 1; // color.x + color.y + color.z > 1, main.cpp:700
         M[3 * p + 0] = keep ? c[0] : 0.0f;
         M[3 * p + 1] = keep ? c[1] : 0.0f;
         M[3 * p + 2] = keep ? c[2] : 0.0f;
-        if (x == 0) progress[y] = 0;
+        if (x == 0) progress[v * H + y] = 0;
+        if (p == 0) progress[(size_t)nViews * H] = 0;
     }
 }
 #define BLOOM_R 10
 #define BLOOM_D (2 * BLOOM_R + 1)
-__global__ void __launch_bounds__(128) k_bloom(float* M, const float* __restrict__ frame, int W, int H, float* __restrict__ out,
-                                               int* progress)
+// A block takes its (view, group of 4 rows) from a ticket, not from blockIdx: row y waits only on row y - 1 of its view, which
+// is in the same block or in a block holding a smaller ticket - a block that has started and so will finish. No wait depends on
+// the order in which blocks are dispatched or on how many are resident.
+__global__ void __launch_bounds__(128) k_bloom(float* M, const float* __restrict__ frame, int W, int H, int nViews,
+                                               float* __restrict__ out, int* progress)
 {
     __shared__ float win[4][3][BLOOM_D][BLOOM_D]; // [warp][channel][window row i + 10][column mod 21]
+    __shared__ int ticket;
+    if (threadIdx.x == 0) ticket = atomicAdd(progress + (size_t)nViews * H, 1);
+    __syncthreads();
+    const int groups = (H + 3) / 4, v = ticket / groups;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int y = blockIdx.x * 4 + warp;
+    const int y = (ticket - v * groups) * 4 + warp;
     if (y >= H) return;
+    const size_t vOff = (size_t)v * W * H * 3;
+    M += vOff;
+    frame += vOff;
+    out += vOff;
+    progress += (size_t)v * H;
     float(*w)[BLOOM_D][BLOOM_D] = win[warp];
     const int i0 = y - BLOOM_R < 0 ? -y : -BLOOM_R, i1 = y + BLOOM_R > H - 1 ? H - 1 - y : BLOOM_R; // valid rows of the window
     int seen = y == 0 ? W : 0; // columns of row y - 1 known to be finished
@@ -2142,18 +2183,24 @@ __global__ void __launch_bounds__(128) k_bloom(float* M, const float* __restrict
         __syncwarp();
     }
 }
-void launchBloom(const float* frame, int W, int H, float* M, int* progress, float* out, int numSMs, cudaStream_t st)
+void launchBloom(const float* frame, int W, int H, int nViews, float* M, int* progress, float* out, int numSMs, cudaStream_t st)
 {
-    const size_t n = (size_t)W * H;
+    const size_t n = (size_t)W * H * nViews;
     int blocks = (int)((n + 255) / 256);
     blocks = blocks > numSMs * 16 ? numSMs * 16 : blocks;
-    k_bloom_init<<<blocks, 256, 0, st>>>(frame, W, H, M, progress);
-    k_bloom<<<(H + 3) / 4, 128, 0, st>>>(M, frame, W, H, out, progress);
+    k_bloom_init<<<blocks, 256, 0, st>>>(frame, W, H, nViews, M, progress);
+    k_bloom<<<nViews * ((H + 3) / 4), 128, 0, st>>>(M, frame, W, H, nViews, out, progress);
 }
 
-void launchAADownsample(const float* big, int W, int H, float* out, cudaStream_t st)
+void launchAADownsample(const float* big, int W, int H, int nViews, float* out, cudaStream_t st)
 {
-    k_aa_downsample<<<(W * H + 255) / 256, 256, 0, st>>>(big, W, H, out);
+    const size_t n = (size_t)W * H * nViews;
+    k_aa_downsample<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(big, W, H, nViews, out);
+}
+void launchBlurViews(const float* frames, int c0, int c1, size_t n, const float* bloomIn, float* acc, float div, cudaStream_t st)
+{
+    const size_t total = (size_t)((c1 - 1) / 15 - c0 / 15 + 1) * n;
+    if (total) k_blur_views<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(frames, c0, c1, n, bloomIn, acc, div);
 }
 void launchAccumulate(float* acc, const float* frame, size_t n, bool first, cudaStream_t st)
 {

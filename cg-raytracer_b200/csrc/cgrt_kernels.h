@@ -259,8 +259,13 @@ void launchAssemble(const float* gathered, size_t perRankFloats, const int* tile
                     cudaStream_t st);
 void launchFlagSignal(uint32_t* const* flags, int n, uint32_t seq, cudaStream_t st);
 void launchFlagWait(const uint32_t* flags, int n, uint32_t seq, unsigned long long timeoutNs, uint32_t* status, cudaStream_t st);
-void launchBloom(const float* frame, int W, int H, float* M, int* progress, float* out, int numSMs, cudaStream_t st);
-void launchAADownsample(const float* big, int W, int H, float* out, cudaStream_t st);
+// bloom of nViews frames [nViews][H][W][3] into out (same layout); M: nViews x W x H x 3 floats, progress: nViews x H + 1 ints
+void launchBloom(const float* frame, int W, int H, int nViews, float* M, int* progress, float* out, int numSMs, cudaStream_t st);
+// big [nViews][2H][2W][3] -> out [nViews][H][W][3]
+void launchAADownsample(const float* big, int W, int H, int nViews, float* out, cudaStream_t st);
+// motion blur of several views: frames holds cameras c0..c1-1 of the flattened (view, k) list (15 per view, view-major), each
+// W x H x 3 floats; acc = [views][W x H x 3]. bloomIn (optional): the un-shifted frames, whose bloom output acc holds before k = 0.
+void launchBlurViews(const float* frames, int c0, int c1, size_t n, const float* bloomIn, float* acc, float div, cudaStream_t st);
 void launchAccumulate(float* acc, const float* frame, size_t n, bool first, cudaStream_t st);
 void launchDivide(const float* acc, size_t n, float div, float* out, cudaStream_t st);
 void launchQuantize(const float* frame, size_t nPixels, uint8_t* rgba, cudaStream_t st);

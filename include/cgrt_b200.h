@@ -307,6 +307,30 @@ int cgrt_render_collect_stats(cgrt_scene* s, cgrt_render_stats* stats);
 #define CGRT_EFFECT_BLOOM 4
 int cgrt_render_effects(cgrt_scene* s, const cgrt_camera* cam, const cgrt_render_params* p, int32_t effects, float* rgb,
                         cgrt_render_stats* stats);
+/* The effects of cgrt_render_effects for several views of one scene in one call, on the caller's stream (turntables, datasets,
+ * a UI that keeps its frames on the GPU). Every render inside the call is one frame of a views batch (cgrt_render_views) of at
+ * most 2^25 pixel slots: the 15 motion-blur cameras of as many whole views as fit (a view whose 15 cameras do not fit, e.g. 4K,
+ * spreads them over several batches in order), the un-shifted views of bloom, the 2W x 2H views of anti-aliasing. One kernel
+ * adds each batch's motion-blur frames into the views' running sums, one bloom pass runs the row recurrences of all views.
+ *   Output   rgb / d_out = [n_views][H][W][3], each view in Screen layout (row H-1-y).
+ *   Equality view v is bit for bit what cgrt_render_effects(s, &cams[v], p, effects, ...) returns, for every accepted
+ *            combination of effects, with spherical-light soft shadows too, and at trace limit 0. effects == 0 is
+ *            cgrt_render_views.
+ *   Stats    primary, primary_hit, shadow and bounce are the sums of those calls' statistics; kernel_launches counts every
+ *            launch of this call; device_ms runs from the call's first event to its last; pipeline is that of the last
+ *            render; no per-class times (there is no profiling mode).
+ *   Refused  (CGRT_ERR_INVALID): what cgrt_render_effects refuses for one view (unknown effect bits, bloom with
+ *            anti-aliasing, 4 x width x height > 2^28 for anti-aliasing, a frame too tall for the bloom pass) and, before any
+ *            CUDA call, null cams / rgb / d_out, n_views outside 1..1024, n_views x width x height > 2^28, world != 1, any
+ *            p->flags other than 0.
+ * The scene's effect buffers grow with the call and stay. The _device form is asynchronous on `stream`: after the stream has
+ * synchronised, cgrt_render_collect_stats returns the sums above for the whole call (CGRT_ERR_CUDA if the persistent
+ * wavefront's watchdog fired in any of its renders). Frames of one scene are enqueued on one stream or ordered by the caller.
+ * The host form is the device form on the scene's stream, one copy to rgb and one synchronisation. */
+int cgrt_render_effects_views(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, const cgrt_render_params* p,
+                              int32_t effects, float* rgb, cgrt_render_stats* stats);
+int cgrt_render_effects_views_device(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, const cgrt_render_params* p,
+                                     int32_t effects, float* d_out, void* stream);
 /* Streaming form of cgrt_render for hosts that render frame after frame (the reference re-renders every UI frame in
  * ViewMode::RayTracing, src/main.cpp:907-914): cgrt_render_submit enqueues the frame (per-frame camera + lights upload, the
  * kernels, the device->host copy into rgb_host) and returns; up to two frames are in flight, so the copy of frame k overlaps
