@@ -85,7 +85,7 @@ EXPORTS = [
     "cgrt_flag_signal", "cgrt_flag_wait", "cgrt_bvh_fast_tree_stats", "cgrt_render_submit", "cgrt_render_wait",
     "cgrt_render_effects", "cgrt_scene_set_spherical_lights", "cgrt_debug_wave_timeline", "cgrt_debug_wave_tuner",
     "cgrt_render_views", "cgrt_render_views_device", "cgrt_render_aovs", "cgrt_render_aovs_device",
-    "cgrt_render_effects_views", "cgrt_render_effects_views_device",
+    "cgrt_render_effects_views", "cgrt_render_effects_views_device", "cgrt_render_lights", "cgrt_render_lights_device",
 ]
 
 _lib = None
@@ -138,6 +138,9 @@ def load_library(path=None):
         "cgrt_render_aovs": (C.c_int, [vp, C.POINTER(Camera), i32, C.POINTER(RenderParams), vp, C.POINTER(AovBuffers),
                                         C.POINTER(RenderStats)]),
         "cgrt_render_aovs_device": (C.c_int, [vp, C.POINTER(Camera), i32, C.POINTER(RenderParams), vp, C.POINTER(AovBuffers), vp]),
+        "cgrt_render_lights": (C.c_int, [vp, C.POINTER(Camera), i32, C.POINTER(RenderParams), i32p, i32, i32, vp, vp,
+                                          C.POINTER(RenderStats)]),
+        "cgrt_render_lights_device": (C.c_int, [vp, C.POINTER(Camera), i32, C.POINTER(RenderParams), i32p, i32, i32, vp, vp, vp]),
         "cgrt_render_collect_stats": (C.c_int, [vp, C.POINTER(RenderStats)]),
         "cgrt_tile_buffer_floats": (sz, [C.POINTER(RenderParams)]),
         "cgrt_tile_list": (C.c_int, [C.POINTER(RenderParams), i32, i32p, i32]),
@@ -267,6 +270,7 @@ class Scene:
         h = C.c_void_p()
         check(self.lib.cgrt_scene_create(C.byref(d), C.byref(o), C.byref(h)))
         self.h = h
+        self.n_point_lights = self.n_spherical_lights = 0  # as set_lights / set_spherical_lights gave them (render_lights' groups)
         if lights is not None:
             self.set_lights(lights)
 
@@ -284,11 +288,13 @@ class Scene:
     def set_lights(self, lights):
         l = np.ascontiguousarray(lights, np.float32).reshape(-1, 6)
         check(self.lib.cgrt_scene_set_lights(self.h, _fp(l), l.shape[0]))
+        self.n_point_lights = l.shape[0]
 
     def set_spherical_lights(self, lights, seed=1):
         """Scene::sphericalLight: [n][7] = position, radius, colour (soft shadows of main.cpp:168-218)."""
         l = np.ascontiguousarray(lights, np.float32).reshape(-1, 7)
         check(self.lib.cgrt_scene_set_spherical_lights(self.h, _fp(l), l.shape[0], seed))
+        self.n_spherical_lights = l.shape[0]
 
     def set_spheres(self, spheres):
         s = np.ascontiguousarray(spheres, np.float32).reshape(-1, 12)
@@ -431,10 +437,45 @@ class Scene:
         check(self.lib.cgrt_render_aovs_device(self.h, arr, len(cams), C.byref(params), C.c_void_p(d_rgb_ptr), C.byref(a),
                                                C.c_void_p(stream_ptr)))
 
+    def render_lights(self, cams, W, H, trace_limit=2, groups=None, n_groups=None):
+        """cgrt_render_lights: (rgb[K,H,W,3], light_rgb[G,K,H,W,3], stats dict summed over the views), Screen layout.
+        groups: each light's group (point lights, then spherical lights; -1 = in no group); default one group per light in
+        that order. n_groups: G, default max(groups) + 1. Group g is bit for bit the frame with every light outside g black."""
+        n = self.n_point_lights + self.n_spherical_lights
+        lg = np.ascontiguousarray(np.arange(n) if groups is None else groups, np.int32)
+        G = int(n_groups if n_groups is not None else max(int(lg.max(initial=-1)) + 1, 1))
+        K = len(cams)
+        arr = (Camera * K)(*cams)
+        p = render_params(W, H, trace_limit)
+        rgb = np.zeros((K, H, W, 3), np.float32)
+        light_rgb = np.zeros((G, K, H, W, 3), np.float32)
+        st = RenderStats()
+        check(self.lib.cgrt_render_lights(self.h, arr, K, C.byref(p), lg.ctypes.data_as(C.POINTER(C.c_int32)), len(lg), G,
+                                          _vp(rgb), _vp(light_rgb), C.byref(st)))
+        return rgb, light_rgb, st.as_dict()
+
+    def render_lights_device(self, cams, params, groups, n_groups, d_rgb_ptr, d_groups_ptr, stream_ptr=0):
+        """Device form: rgb [K][H][W][3] into d_rgb_ptr and the groups [n_groups][K][H][W][3] into d_groups_ptr on the stream;
+        groups is the host list of each light's group. Statistics through collect_stats()."""
+        arr = (Camera * len(cams))(*cams)
+        lg = np.ascontiguousarray(groups, np.int32)
+        check(self.lib.cgrt_render_lights_device(self.h, arr, len(cams), C.byref(params), lg.ctypes.data_as(C.POINTER(C.c_int32)),
+                                                 len(lg), n_groups, C.c_void_p(d_rgb_ptr), C.c_void_p(d_groups_ptr),
+                                                 C.c_void_p(stream_ptr)))
+
     def collect_stats(self):
         st = RenderStats()
         check(self.lib.cgrt_render_collect_stats(self.h, C.byref(st)))
         return st.as_dict()
+
+
+def relight(light_rgb, gains):
+    """sum_g gains[g] * light_rgb[g]: the frame with group g's light colours scaled by gains[g] ([G][3], per channel), from the
+    buffers of Scene.render_lights without tracing again. Approximate: it matches a render with the scaled colours only up to
+    float rounding (the render scales each light before summing, this scales the group's sum)."""
+    light_rgb = np.asarray(light_rgb, np.float32)
+    g = np.asarray(gains, np.float32).reshape(light_rgb.shape[0], 1, 1, 1, 3)
+    return (light_rgb * g).sum(axis=0, dtype=np.float32)
 
 
 # -- unit predicates (src/ray_tracing.h:10-20), batched, host buffers ---------------------------------------------------

@@ -292,7 +292,7 @@ struct cgrt_scene {
     DevBuf<int> pathPix, counts, tileList;
     DevBuf<unsigned long long> tests;
     DevBuf<float4> hitRec;
-    DevBuf<float> aovStage; // cgrt_render_aovs: the requested per-pixel buffers on the device before their copy to the host
+    DevBuf<float> aovStage; // cgrt_render_aovs / cgrt_render_lights: their per-pixel buffers on the device before the copy to the host
     DevBuf<int> hitList, pathDepth, replayShadow;
     DevBuf<float4> replayQ;
     DevBuf<float4> cRay[2], cRes[2], sRay[2], sRes[2];
@@ -1448,10 +1448,26 @@ static int waveQueues(cgrt_scene* s, cudaStream_t st, WaveQ& Q)
     return CGRT_OK;
 }
 
-// one frame of nViews cameras into d_out (cgrt_render_device: one camera; cgrt_render_views_device: several); aov (optional,
-// whole frames of the path, round or wave pipeline only): the per-pixel buffers of cgrt_render_aovs
+// cgrt_render_lights' groups: lightGroup[nLights] (host; point lights, then spherical lights) and the device buffers
+struct LightGroups {
+    const int32_t* lightGroup;
+    int nLights;
+    LightGroupBuffers out;
+};
+
+// the w lane of light i's colour in the parameter block: its group (bit-cast int) in a frame with light groups, else 0
+static float groupLane(const LightGroups* lg, size_t i)
+{
+    float f = 0.0f;
+    if (lg) std::memcpy(&f, lg->lightGroup + i, sizeof f);
+    return f;
+}
+
+// one frame of nViews cameras into d_out (cgrt_render_device: one camera; cgrt_render_views_device: several); aov and lg (optional,
+// whole frames of the path, round or wave pipeline only): the per-pixel buffers of cgrt_render_aovs, the light groups of
+// cgrt_render_lights
 static int renderDevice(cgrt_scene* s, const cgrt_camera* cams, int nViews, const cgrt_render_params* p, float* d_out, void* stream,
-                        const AovBuffers* aov = nullptr)
+                        const AovBuffers* aov = nullptr, const LightGroups* lg = nullptr)
 {
     RC(useSceneDevice(s));
     std::lock_guard<std::mutex> lk(s->mu);
@@ -1463,6 +1479,8 @@ static int renderDevice(cgrt_scene* s, const cgrt_camera* cams, int nViews, cons
     RC(prepareFrame(s, cams, nViews, p, P, &dTiles, &dSeq, &pipe));
     if (P.screenLayout && P.world > 1 && pipe == PIPE_COUNT)
         return fail(CGRT_ERR_INVALID, "CGRT_RENDER_COUNT renders into the tile-major buffer; it cannot be combined with CGRT_RENDER_SCREEN_LAYOUT");
+    // the lights may have changed since the caller's arguments were checked
+    if (lg && lg->nLights != P.nLights + P.nSph) return fail(CGRT_ERR_INVALID, "n_lights does not match the scene's lights");
     // per-frame upload (camera constants + lights, read live from the scene like src/main.cpp:835-876 allows)
     // the slot's previous frame may still be waiting for its copy (frames enqueued faster than the stream runs them)
     cudaEvent_t& copied = s->ringCopied[s->ringPos];
@@ -1475,12 +1493,12 @@ static int renderDevice(cgrt_scene* s, const cgrt_camera* cams, int nViews, cons
     for (size_t i = 0; i < s->lights.size(); i++) {
         const cgrt_point_light& l = s->lights[i];
         hl[2 * i] = make_float4(l.position[0], l.position[1], l.position[2], 0.0f);
-        hl[2 * i + 1] = make_float4(l.color[0], l.color[1], l.color[2], 0.0f);
+        hl[2 * i + 1] = make_float4(l.color[0], l.color[1], l.color[2], groupLane(lg, i));
     }
-    for (int i = 0; i < P.nSph; i++) { // spherical lights follow the point lights: [position | radius] [colour | -]
+    for (int i = 0; i < P.nSph; i++) { // spherical lights follow the point lights: [position | radius] [colour | group]
         const float* q = s->sphLights.data() + 7 * (size_t)i;
         hl[2 * (s->lights.size() + i)] = make_float4(q[0], q[1], q[2], q[3]);
-        hl[2 * (s->lights.size() + i) + 1] = make_float4(q[4], q[5], q[6], 0.0f);
+        hl[2 * (s->lights.size() + i) + 1] = make_float4(q[4], q[5], q[6], groupLane(lg, s->lights.size() + i));
     }
     float4* hc = hl + 2 * (s->lights.size() + (size_t)P.nSph); // the views' cameras follow the lights
     for (int v = 0; v < nViews; v++) {
@@ -1549,6 +1567,14 @@ static int renderDevice(cgrt_scene* s, const cgrt_camera* cams, int nViews, cons
     if (aov)
         launches += launchAovPass(s->dev, dP, P, s->hitRec.p, P.traceLimit > 0 ? s->pathDepth.p : nullptr, pipe == PIPE_PATHS,
                                   s->pathPix.p, s->counts.p, dSeq, *aov, numSMs, st);
+    // the light-group pass, at the same point; the path pipeline's misses and a black frame leave no record
+    if (lg) {
+        if (pipe == PIPE_PATHS || P.traceLimit == 0)
+            CK(cudaMemsetAsync(lg->out.rgb, 0, lg->out.groupFloats * lg->out.nGroups * sizeof(float), st));
+        if (P.traceLimit > 0)
+            launches += launchLightPass(s->dev, dP, P, dLights, s->hitRec.p, s->lit.p, P.nSph ? s->soft.p : nullptr, s->pathDepth.p,
+                                        pipe == PIPE_PATHS, s->pathPix.p, s->counts.p, dSeq, lg->out, numSMs, st);
+    }
     s->lastPipeline = pipe;
     CK(cudaEventRecord(s->ev1, st));
     CK(cudaGetLastError());
@@ -1607,6 +1633,36 @@ int cgrt_render_aovs_device(cgrt_scene* s, const cgrt_camera* cams, int32_t n_vi
     RC(checkAovs(s, cams, n_views, p, d_rgb, d_aov));
     const AovBuffers A = {d_aov->depth, d_aov->tri, d_aov->normal, d_aov->hits};
     return renderDevice(s, cams, n_views, p, d_rgb, stream, &A);
+}
+
+// the arguments cgrt_render_lights refuses: those of cgrt_render_views, null light_group / groups, n_groups outside 1..64, group
+// buffers of more than 2^28 pixels, a light count other than the scene's, and a group index outside -1..n_groups-1
+static int checkLights(cgrt_scene* s, const cgrt_camera* cams, int32_t nViews, const cgrt_render_params* p, const float* rgb,
+                       const int32_t* lightGroup, int32_t nLights, int32_t nGroups, const float* groups)
+{
+    RC(checkViews(s, cams, nViews, p, rgb));
+    if (!lightGroup || !groups) return fail(CGRT_ERR_INVALID, "null light_group or groups");
+    if (nGroups < 1 || nGroups > CGRT_MAX_LIGHT_GROUPS) return fail(CGRT_ERR_INVALID, "n_groups must be in 1..64");
+    if ((int64_t)nGroups * nViews * p->width * p->height > (int64_t)1 << 28)
+        return fail(CGRT_ERR_INVALID, "light groups too large: n_groups x n_views x width x height > 2^28");
+    size_t have;
+    {
+        std::lock_guard<std::mutex> lk(s->mu);
+        have = s->lights.size() + s->sphLights.size() / 7;
+    }
+    if (nLights < 0 || (size_t)nLights != have) return fail(CGRT_ERR_INVALID, "n_lights must be the scene's point plus spherical lights");
+    for (int32_t i = 0; i < nLights; i++)
+        if (lightGroup[i] < -1 || lightGroup[i] >= nGroups) return fail(CGRT_ERR_INVALID, "light_group entries must be in -1..n_groups-1");
+    return CGRT_OK;
+}
+
+int cgrt_render_lights_device(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, const cgrt_render_params* p,
+                              const int32_t* light_group, int32_t n_lights, int32_t n_groups, float* d_rgb, float* d_groups,
+                              void* stream)
+{
+    RC(checkLights(s, cams, n_views, p, d_rgb, light_group, n_lights, n_groups, d_groups));
+    const LightGroups G = {light_group, n_lights, {d_groups, (size_t)n_views * p->width * p->height * 3, n_groups}};
+    return renderDevice(s, cams, n_views, p, d_rgb, stream, nullptr, &G);
 }
 
 // One frame's ray statistics (primary, primary_hit, shadow, bounce, replayed_*, pipeline) into a zeroed *stats: counts = its counters
@@ -1905,6 +1961,31 @@ int cgrt_render_aovs(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, co
     if (aov->tri) CK(cudaMemcpyAsync(aov->tri, A.tri, px * sizeof(int32_t), cudaMemcpyDeviceToHost, s->stream));
     if (aov->normal) CK(cudaMemcpyAsync(aov->normal, A.normal, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, s->stream));
     if (aov->hits) CK(cudaMemcpyAsync(aov->hits, A.hits, px, cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaStreamSynchronize(s->stream));
+    if (stats) RC(cgrt_render_collect_stats(s, stats));
+    return CGRT_OK;
+}
+
+// ---- each light group's share of the frame --------------------------------------------------------------------------------------
+int cgrt_render_lights(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, const cgrt_render_params* p,
+                       const int32_t* light_group, int32_t n_lights, int32_t n_groups, float* rgb, float* groups,
+                       cgrt_render_stats* stats)
+{
+    RC(checkLights(s, cams, n_views, p, rgb, light_group, n_lights, n_groups, groups));
+    RC(useSceneDevice(s));
+    std::lock_guard<std::mutex> hostLock(s->hostMu);
+    const size_t px = (size_t)n_views * p->width * p->height;
+    float* stage = nullptr;
+    {
+        std::lock_guard<std::mutex> lk(s->mu);
+        RC(s->frame.ensure(px * 3));
+        RC(s->aovStage.ensure(px * 3 * n_groups));
+        stage = s->aovStage.p;
+    }
+    const LightGroups G = {light_group, n_lights, {stage, px * 3, n_groups}};
+    RC(renderDevice(s, cams, n_views, p, s->frame.p, s->stream, nullptr, &G));
+    CK(cudaMemcpyAsync(rgb, s->frame.p, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaMemcpyAsync(groups, stage, px * 3 * n_groups * sizeof(float), cudaMemcpyDeviceToHost, s->stream));
     CK(cudaStreamSynchronize(s->stream));
     if (stats) RC(cgrt_render_collect_stats(s, stats));
     return CGRT_OK;

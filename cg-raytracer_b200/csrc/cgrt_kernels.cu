@@ -1006,9 +1006,12 @@ __global__ void __launch_bounds__(128, CGRT_MINBLOCKS) k_shadow_replay(DevScene 
 // CG: the lit flags were written by other SMs during this kernel (persistent wavefront): read them through L2
 // nSph / soft: spherical lights (main.cpp:168-218) come first in the sum: (diffuse + specular of a point light at the centre)
 // times the fraction of the light's 200 sample rays that arrive (k_soft_shadows)
-template <bool CG = false>
+// GROUP (the light-group pass): only the lights whose colour's w lane (bit-cast int) is `group`; the others are skipped before
+// any work. A light of colour 0 adds +-0 to a sum that is never -0, so skipping it leaves the same bits.
+template <bool CG = false, bool GROUP = false>
 RT_DEV V3 directColour(const DevScene& S, const float4* __restrict__ lights, int nL, const float4& a, const float4& b,
-                       const float4& c, const uint8_t* __restrict__ lit, V3& ks, int nSph = 0, const float* __restrict__ soft = nullptr)
+                       const float4& c, const uint8_t* __restrict__ lit, V3& ks, int nSph = 0, const float* __restrict__ soft = nullptr,
+                       int group = 0)
 {
     const V3 P = mk3(a), N = mk3(b), D = mk3(c);
     const int mat = f2i(a.w);
@@ -1019,6 +1022,7 @@ RT_DEV V3 directColour(const DevScene& S, const float4* __restrict__ lights, int
     const float shininess = m0.w;
     V3 result = mk3(0.0f, 0.0f, 0.0f);
     for (int l = 0; l < nSph; l++) {
+        if (GROUP && f2i(__ldg(lights + 2 * (nL + l) + 1).w) != group) continue;
         const V3 lightPos = mk3(__ldg(lights + 2 * (nL + l))), lightCol = mk3(__ldg(lights + 2 * (nL + l) + 1));
         const V3 fromPosToLight = normalize3(lightPos - P);
         V3 diffuse = mk3(0.0f, 0.0f, 0.0f), specular = diffuse;
@@ -1032,6 +1036,7 @@ RT_DEV V3 directColour(const DevScene& S, const float4* __restrict__ lights, int
         result = result + specular * softShadowCounter;
     }
     for (int l = 0; l < nL; l++) {
+        if (GROUP && f2i(__ldg(lights + 2 * l + 1).w) != group) continue;
         const V3 lightPos = mk3(__ldg(lights + 2 * l)), lightCol = mk3(__ldg(lights + 2 * l + 1));
         const V3 fromPosToLight = normalize3(lightPos - P);
         if (!(CG ? __ldcg(lit + l) : lit[l])) continue;
@@ -1940,6 +1945,58 @@ __global__ void __launch_bounds__(128) k_aov_paths(DevScene S, const FrameParams
         storeAov(S, A, pathPix[path], pathDepth[path], hitRec + 3 * (size_t)path * levels);
 }
 
+// ---- light groups (cgrt_render_lights) from the hit records, lit flags and soft-shadow fractions the frame left -----------------
+// Per group, the shading of k_shade_slots / k_shade_paths / k_wave phase C with the same arithmetic, restricted to the group's
+// lights: directColour of every level, then the recursion unwound innermost first. A chain of depth 0 (a miss) is +0.
+RT_DEV void storeLightGroups(const DevScene& S, const FrameParams& P, const float4* __restrict__ lights,
+                             const float4* __restrict__ hitRec, const uint8_t* __restrict__ lit, const float* __restrict__ soft,
+                             int chain, int depth, int outIdx, const LightGroupBuffers& G)
+{
+    const int nL = P.nLights, levels = P.traceLimit > 1 ? P.traceLimit : 1;
+    for (int g = 0; g < G.nGroups; g++) {
+        V3 colour = mk3(0.0f, 0.0f, 0.0f);
+        if (depth > 0) {
+            V3 direct[CGRT_MAX_LEVELS], ksv[CGRT_MAX_LEVELS];
+            for (int k = 0; k < depth; k++) {
+                const int rec = chain * levels + k;
+                const float4* r = hitRec + 3 * (size_t)rec;
+                direct[k] = directColour<false, true>(S, lights, nL, r[0], r[1], r[2], lit + (size_t)rec * nL, ksv[k], P.nSph,
+                                                      P.nSph ? soft + (size_t)rec * P.nSph : nullptr, g);
+            }
+            int k = depth - 1;
+            colour = (ksv[k].z <= 0.01f) ? direct[k] : direct[k] + mk3(0.0f, 0.0f, 0.0f) * ksv[k];
+            for (k = depth - 2; k >= 0; k--) colour = direct[k] + colour * ksv[k];
+        }
+        storeRGB(G.rgb + (size_t)g * G.groupFloats, outIdx, colour);
+    }
+}
+
+// one thread per pixel slot (k_wave and the round pipeline: one record chain per slot; padding slots write nothing)
+__global__ void __launch_bounds__(128) k_light_slots(DevScene S, const FrameParams* __restrict__ Pp, const float4* __restrict__ lights,
+                                                     const float4* __restrict__ hitRec, const uint8_t* __restrict__ lit,
+                                                     const float* __restrict__ soft, const int* __restrict__ pathDepth,
+                                                     const int2* __restrict__ tileSeq, LightGroupBuffers G)
+{
+    const FrameParams P = *Pp;
+    for (int slot = blockIdx.x * blockDim.x + threadIdx.x; slot < P.nSlots; slot += gridDim.x * blockDim.x) {
+        int x, y, outIdx, local;
+        if (!seqToPixel(P, tileSeq, slot, x, y, outIdx, local)) continue;
+        storeLightGroups(S, P, lights, hitRec, lit, soft, slot, pathDepth[slot], outIdx, G);
+    }
+}
+
+// path pipeline: one thread per path (primary rays that hit), into group buffers already cleared to +0
+__global__ void __launch_bounds__(128) k_light_paths(DevScene S, const FrameParams* __restrict__ Pp, const float4* __restrict__ lights,
+                                                     const float4* __restrict__ hitRec, const uint8_t* __restrict__ lit,
+                                                     const int* __restrict__ pathDepth, const int* __restrict__ pathPix,
+                                                     const int* __restrict__ counts, LightGroupBuffers G)
+{
+    const FrameParams P = *Pp;
+    const int n = counts[CGRT_CNT_PATHS];
+    for (int path = blockIdx.x * blockDim.x + threadIdx.x; path < n; path += gridDim.x * blockDim.x)
+        storeLightGroups(S, P, lights, hitRec, lit, nullptr, path, pathDepth[path], pathPix[path], G);
+}
+
 // ---- synchronous host render, overlapped delivery: the bounding box of the pixels the shading pass coloured (counts[CGRT_CNT_BBOX],
 // kept by the shading pass), copied from the device frame straight into the caller's page-locked frame in full 128-byte runs;
 // every other pixel of that frame was blanked by a copy-engine transfer while the frame rendered
@@ -2588,6 +2645,18 @@ int launchAovPass(const DevScene& S, const FrameParams* dP, const FrameParams& h
     k_aov_slots<<<grid, 128, 0, st>>>(S, dP, hitRec, nullptr, dTileSeq, A); // the misses have no record
     k_aov_paths<<<grid, 128, 0, st>>>(S, dP, hitRec, pathDepth, pathPix, counts, A);
     return 2;
+}
+
+int launchLightPass(const DevScene& S, const FrameParams* dP, const FrameParams& hP, const float4* dLights, const float4* hitRec,
+                    const uint8_t* lit, const float* soft, const int* pathDepth, bool perPath, const int* pathPix, const int* counts,
+                    const int2* dTileSeq, const LightGroupBuffers& G, int numSMs, cudaStream_t st)
+{
+    const int grid = gridFor((size_t)hP.nSlots, 128, numSMs * 16);
+    if (perPath)
+        k_light_paths<<<grid, 128, 0, st>>>(S, dP, dLights, hitRec, lit, pathDepth, pathPix, counts, G);
+    else
+        k_light_slots<<<grid, 128, 0, st>>>(S, dP, dLights, hitRec, lit, soft, pathDepth, dTileSeq, G);
+    return 1;
 }
 
 void launchAssemble(const float* gathered, size_t perRankFloats, const int* tileLists, const int* tileCounts, int maxTiles,

@@ -164,6 +164,15 @@ struct AovBuffers {
     uint8_t* hits;  // levels of the pixel's path that recorded a hit (pathDepth)
 };
 
+// Light-group buffers of a frame (cgrt_render_lights): group g's [n_views][H][W][3] at rgb + g * groupFloats, Screen layout.
+// A light's group is the bit-cast int in the w lane of its colour in the parameter block (-1: no group); no other pass reads it.
+struct LightGroupBuffers {
+    float* rgb;
+    size_t groupFloats; // 3 x pixels of all views
+    int nGroups;
+};
+#define CGRT_MAX_LIGHT_GROUPS 64
+
 // ---- persistent wavefront (cgrt_wave.cuh): control block + ticket queue of the single-kernel frame ----------------------------
 #define WCTL_PENDING 0  // u64 at int index 0: (CTAs done with phase A << 32) | rays in flight
 #define WCTL_ERR 2      // watchdog: a warp waited longer than WaveQ::timeoutNs
@@ -253,6 +262,13 @@ int launchWavePipeline(const DevScene& S, const FrameParams* dP, const FramePara
 int launchAovPass(const DevScene& S, const FrameParams* dP, const FrameParams& hP, const float4* hitRec, const int* pathDepth,
                   bool perPath, const int* pathPix, const int* counts, const int2* dTileSeq, const AovBuffers& A, int numSMs,
                   cudaStream_t st);
+// The light-group pass after a frame of the path, round or wave pipeline with trace limit > 0 (whole frames in Screen layout).
+// perPath: the path pipeline's records, written through pathPix into buffers the caller has cleared to +0 (misses have no
+// record); else every pixel slot's chain, misses included. soft: the round pipeline's soft-shadow fractions (spherical lights).
+// Returns the kernels it launched.
+int launchLightPass(const DevScene& S, const FrameParams* dP, const FrameParams& hP, const float4* dLights, const float4* hitRec,
+                    const uint8_t* lit, const float* soft, const int* pathDepth, bool perPath, const int* pathPix, const int* counts,
+                    const int2* dTileSeq, const LightGroupBuffers& G, int numSMs, cudaStream_t st);
 void launchDeliverBox(const int* bbox, int W, int H, const float* frame, float* hostFrame, int numSMs, cudaStream_t st);
 void launchAssemble(const float* gathered, size_t perRankFloats, const int* tileLists, const int* tileCounts, int maxTiles,
                     int world, int tileW, int tileH, int tilesX, int width, int height, float* frame, int numSMs,

@@ -285,6 +285,39 @@ int cgrt_render_aovs(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, co
                      const cgrt_aov_buffers* aov, cgrt_render_stats* stats);
 int cgrt_render_aovs_device(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, const cgrt_render_params* p,
                             float* d_rgb, const cgrt_aov_buffers* d_aov, void* stream);
+/* Light groups: cgrt_render_views with each group's share of every pixel in its own buffer, so that a light's colour can be
+ * edited (relit) without tracing the frame again. One pass after the frame shades the hit records, lit flags and soft-shadow
+ * fractions the frame left once per group, with the frame's arithmetic, restricted to the group's lights (DESIGN.md 4.5).
+ *   Groups   light_group[n_lights] (host memory, read before the call returns) gives each light's group: the scene's point
+ *            lights in cgrt_scene_set_lights order, then its spherical lights in cgrt_scene_set_spherical_lights order. An
+ *            entry is a group 0..n_groups-1, or -1: the light is in no group (it lights rgb, no group buffer). n_groups is
+ *            1..64; a group without lights is +0 everywhere.
+ *   Layout   groups is [n_groups][n_views][H][W][3], each view in Screen layout (row H-1-y) like rgb.
+ *   Equality rgb is bit for bit what cgrt_render_views returns for the same arguments; so are the stats, except
+ *            kernel_launches, which also counts the group pass (device_ms covers it).
+ *   Exact    (1) group g of view v is bit for bit view v of cgrt_render_views with every light outside g given colour
+ *            (0,0,0), positions, radii, the spherical-light seed and the order of the lights unchanged (soft-shadow samples
+ *            are keyed by the light's index, which does not change). (2) So a group holding every light equals rgb bit for
+ *            bit. Reason: a light of colour 0 adds +-0 to a sum that is never -0, and the pass skips it. Precondition:
+ *            finite material values and light colours, and shininess >= 0 (every preset and fixture meets it).
+ *   Approx.  (3) the sum of the groups plus the share of the lights in no group equals rgb up to float reassociation
+ *            only: a pixel sums its lights in one order, the groups split that sum. Scaling a group buffer by a colour gain
+ *            likewise matches a render with that light colour scaled up to rounding.
+ *   Limit 0  the frame traces nothing: every group buffer is +0.
+ *   Refused  (CGRT_ERR_INVALID, before any CUDA call): everything cgrt_render_views refuses (so whole frames only, no
+ *            CGRT_RENDER_COUNT, no CGRT_RENDER_SCREEN_LAYOUT), a null light_group or groups, n_groups outside 1..64,
+ *            n_groups x n_views x W x H > 2^28, n_lights other than the scene's point plus spherical lights (checked again
+ *            when the frame reads the lights, which may change in between), and an entry outside -1..n_groups-1.
+ * The host form stages the group buffers on the device, copies rgb and them back on the scene's stream and synchronises once.
+ * The _device form takes device pointers and is asynchronous on `stream`; its statistics come from cgrt_render_collect_stats.
+ * Measured on one B200 (1000 W power limit): one group adds 0.034-0.050 ms to a 1080p frame (C3, trace limit 5: 1.077 vs
+ * 1.127 ms, DESIGN.md 4.5). */
+int cgrt_render_lights(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, const cgrt_render_params* p,
+                       const int32_t* light_group, int32_t n_lights, int32_t n_groups, float* rgb, float* groups,
+                       cgrt_render_stats* stats);
+int cgrt_render_lights_device(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, const cgrt_render_params* p,
+                              const int32_t* light_group, int32_t n_lights, int32_t n_groups, float* d_rgb, float* d_groups,
+                              void* stream);
 int cgrt_render_collect_stats(cgrt_scene* s, cgrt_render_stats* stats);
 /* renderRayTracing's optional passes around the path (UI toggles, default off, src/main.cpp:33-35):
  *   CGRT_EFFECT_ANTIALIAS   src/main.cpp:663-687: four rays per pixel = the pixel-corner rays of the (2W x 2H) frame, summed in
