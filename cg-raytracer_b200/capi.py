@@ -72,6 +72,14 @@ class AovBuffers(C.Structure):
     _fields_ = [("depth", C.c_void_p), ("tri", C.c_void_p), ("normal", C.c_void_p), ("hits", C.c_void_p)]
 
 
+class PathBuffers(C.Structure):
+    """cgrt_path_buffers: every level of each pixel's mirror path (host or device pointers; None = not produced)."""
+    _fields_ = [("ray", C.c_void_p), ("depth", C.c_void_p), ("tri", C.c_void_p), ("normal", C.c_void_p), ("position", C.c_void_p),
+                ("visibility", C.c_void_p)]
+
+
+PATH_KEYS = ("ray", "depth", "tri", "normal", "position", "visibility")
+
 EXPORTS = [
     "cgrt_version", "cgrt_last_error", "cgrt_device_count", "cgrt_scene_create", "cgrt_scene_destroy",
     "cgrt_scene_set_lights", "cgrt_scene_set_spheres", "cgrt_bvh_num_levels", "cgrt_bvh_num_nodes",
@@ -86,6 +94,7 @@ EXPORTS = [
     "cgrt_render_effects", "cgrt_scene_set_spherical_lights", "cgrt_debug_wave_timeline", "cgrt_debug_wave_tuner",
     "cgrt_render_views", "cgrt_render_views_device", "cgrt_render_aovs", "cgrt_render_aovs_device",
     "cgrt_render_effects_views", "cgrt_render_effects_views_device", "cgrt_render_lights", "cgrt_render_lights_device",
+    "cgrt_render_paths", "cgrt_render_paths_device",
 ]
 
 _lib = None
@@ -141,6 +150,10 @@ def load_library(path=None):
         "cgrt_render_lights": (C.c_int, [vp, C.POINTER(Camera), i32, C.POINTER(RenderParams), i32p, i32, i32, vp, vp,
                                           C.POINTER(RenderStats)]),
         "cgrt_render_lights_device": (C.c_int, [vp, C.POINTER(Camera), i32, C.POINTER(RenderParams), i32p, i32, i32, vp, vp, vp]),
+        "cgrt_render_paths": (C.c_int, [vp, C.POINTER(Camera), i32, C.POINTER(RenderParams), i32, i32, vp, C.POINTER(PathBuffers),
+                                         C.POINTER(RenderStats)]),
+        "cgrt_render_paths_device": (C.c_int, [vp, C.POINTER(Camera), i32, C.POINTER(RenderParams), i32, i32, vp,
+                                                C.POINTER(PathBuffers), vp]),
         "cgrt_render_collect_stats": (C.c_int, [vp, C.POINTER(RenderStats)]),
         "cgrt_tile_buffer_floats": (sz, [C.POINTER(RenderParams)]),
         "cgrt_tile_list": (C.c_int, [C.POINTER(RenderParams), i32, i32p, i32]),
@@ -270,7 +283,7 @@ class Scene:
         h = C.c_void_p()
         check(self.lib.cgrt_scene_create(C.byref(d), C.byref(o), C.byref(h)))
         self.h = h
-        self.n_point_lights = self.n_spherical_lights = 0  # as set_lights / set_spherical_lights gave them (render_lights' groups)
+        self.n_point_lights = self.n_spherical_lights = 0  # as set_lights / set_spherical_lights gave them (render_lights' groups, render_paths' visibility)
         if lights is not None:
             self.set_lights(lights)
 
@@ -462,6 +475,36 @@ class Scene:
         check(self.lib.cgrt_render_lights_device(self.h, arr, len(cams), C.byref(params), lg.ctypes.data_as(C.POINTER(C.c_int32)),
                                                  len(lg), n_groups, C.c_void_p(d_rgb_ptr), C.c_void_p(d_groups_ptr),
                                                  C.c_void_p(stream_ptr)))
+
+    def render_paths(self, cams, W, H, trace_limit=2, n_levels=None, ray=True, depth=True, tri=True, normal=True, position=True,
+                     visibility=True):
+        """cgrt_render_paths: (rgb[K,H,W,3], {"ray": RAY_DTYPE[Lv,K,H,W], "depth": float32[Lv,K,H,W], "tri": int32[Lv,K,H,W],
+        "normal" / "position": float32[Lv,K,H,W,3], "visibility": float32[Lv,K,H,W,n_lights]} with the requested keys only,
+        stats dict summed over the views). Level l is the ray trace(l) cast and its hit; Screen layout, like rgb. n_levels
+        (Lv): default max(trace_limit, 1). Lights: point lights, then spherical lights."""
+        K = len(cams)
+        Lv = int(n_levels if n_levels is not None else max(trace_limit, 1))
+        nl = self.n_point_lights + self.n_spherical_lights
+        arr = (Camera * K)(*cams)
+        p = render_params(W, H, trace_limit)
+        rgb = np.zeros((K, H, W, 3), np.float32)
+        want = dict(ray=(ray, (Lv, K, H, W), RAY_DTYPE), depth=(depth, (Lv, K, H, W), np.float32), tri=(tri, (Lv, K, H, W), np.int32),
+                    normal=(normal, (Lv, K, H, W, 3), np.float32), position=(position, (Lv, K, H, W, 3), np.float32),
+                    visibility=(visibility, (Lv, K, H, W, nl), np.float32))
+        out = {k: np.zeros(shp, dt) for k, (on, shp, dt) in want.items() if on}
+        b = PathBuffers(*[out[k].ctypes.data if k in out else None for k in PATH_KEYS])
+        st = RenderStats()
+        check(self.lib.cgrt_render_paths(self.h, arr, K, C.byref(p), Lv, nl, _vp(rgb), C.byref(b), C.byref(st)))
+        return rgb, out, st.as_dict()
+
+    def render_paths_device(self, cams, params, n_levels, d_rgb_ptr, d_path_ptrs, stream_ptr=0):
+        """Device form: rgb [K][H][W][3] into d_rgb_ptr and the buffers of d_path_ptrs (dict of device pointers with the keys of
+        render_paths; a missing key or None = not produced) on the stream; statistics through collect_stats()."""
+        arr = (Camera * len(cams))(*cams)
+        b = PathBuffers(*[d_path_ptrs.get(k) for k in PATH_KEYS])
+        check(self.lib.cgrt_render_paths_device(self.h, arr, len(cams), C.byref(params), n_levels,
+                                                self.n_point_lights + self.n_spherical_lights, C.c_void_p(d_rgb_ptr), C.byref(b),
+                                                C.c_void_p(stream_ptr)))
 
     def collect_stats(self):
         st = RenderStats()

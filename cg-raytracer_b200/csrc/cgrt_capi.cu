@@ -292,7 +292,7 @@ struct cgrt_scene {
     DevBuf<int> pathPix, counts, tileList;
     DevBuf<unsigned long long> tests;
     DevBuf<float4> hitRec;
-    DevBuf<float> aovStage; // cgrt_render_aovs / cgrt_render_lights: their per-pixel buffers on the device before the copy to the host
+    DevBuf<float> aovStage; // cgrt_render_aovs / _lights / _paths: their per-pixel buffers on the device before the copy to the host
     DevBuf<int> hitList, pathDepth, replayShadow;
     DevBuf<float4> replayQ;
     DevBuf<float4> cRay[2], cRes[2], sRay[2], sRes[2];
@@ -1480,7 +1480,8 @@ static int renderDevice(cgrt_scene* s, const cgrt_camera* cams, int nViews, cons
     if (P.screenLayout && P.world > 1 && pipe == PIPE_COUNT)
         return fail(CGRT_ERR_INVALID, "CGRT_RENDER_COUNT renders into the tile-major buffer; it cannot be combined with CGRT_RENDER_SCREEN_LAYOUT");
     // the lights may have changed since the caller's arguments were checked
-    if (lg && lg->nLights != P.nLights + P.nSph) return fail(CGRT_ERR_INVALID, "n_lights does not match the scene's lights");
+    if ((lg && lg->nLights != P.nLights + P.nSph) || (aov && aov->nLights >= 0 && aov->nLights != P.nLights + P.nSph))
+        return fail(CGRT_ERR_INVALID, "n_lights does not match the scene's lights");
     // per-frame upload (camera constants + lights, read live from the scene like src/main.cpp:835-876 allows)
     // the slot's previous frame may still be waiting for its copy (frames enqueued faster than the stream runs them)
     cudaEvent_t& copied = s->ringCopied[s->ringPos];
@@ -1562,11 +1563,12 @@ static int renderDevice(cgrt_scene* s, const cgrt_camera* cams, int nViews, cons
         break;
     }
     }
-    // the AOV pass reads the level-0 hit records the frame left (after the round pipeline's chains have joined on st); a black
-    // frame (trace limit 0) leaves no records and a stale pathDepth
+    // the AOV / mirror-path pass reads the hit records, lit flags and soft-shadow fractions the frame left (after the round
+    // pipeline's chains have joined on st); a black frame (trace limit 0) leaves no records and a stale pathDepth
     if (aov)
-        launches += launchAovPass(s->dev, dP, P, s->hitRec.p, P.traceLimit > 0 ? s->pathDepth.p : nullptr, pipe == PIPE_PATHS,
-                                  s->pathPix.p, s->counts.p, dSeq, *aov, numSMs, st);
+        launches += launchAovPass(s->dev, dP, P, dLights, s->hitRec.p, s->lit.p, P.nSph ? s->soft.p : nullptr,
+                                  P.traceLimit > 0 ? s->pathDepth.p : nullptr, pipe == PIPE_PATHS, s->pathPix.p, s->counts.p, dSeq,
+                                  *aov, numSMs, st);
     // the light-group pass, at the same point; the path pipeline's misses and a black frame leave no record
     if (lg) {
         if (pipe == PIPE_PATHS || P.traceLimit == 0)
@@ -1631,7 +1633,7 @@ int cgrt_render_aovs_device(cgrt_scene* s, const cgrt_camera* cams, int32_t n_vi
                             const cgrt_aov_buffers* d_aov, void* stream)
 {
     RC(checkAovs(s, cams, n_views, p, d_rgb, d_aov));
-    const AovBuffers A = {d_aov->depth, d_aov->tri, d_aov->normal, d_aov->hits};
+    const AovBuffers A = {d_aov->depth, d_aov->tri, d_aov->normal, d_aov->hits, nullptr, nullptr, nullptr, 1, 0, -1};
     return renderDevice(s, cams, n_views, p, d_rgb, stream, &A);
 }
 
@@ -1663,6 +1665,44 @@ int cgrt_render_lights_device(cgrt_scene* s, const cgrt_camera* cams, int32_t n_
     RC(checkLights(s, cams, n_views, p, d_rgb, light_group, n_lights, n_groups, d_groups));
     const LightGroups G = {light_group, n_lights, {d_groups, (size_t)n_views * p->width * p->height * 3, n_groups}};
     return renderDevice(s, cams, n_views, p, d_rgb, stream, nullptr, &G);
+}
+
+// the arguments cgrt_render_paths refuses: those of cgrt_render_views, a null paths or one that requests no buffer, n_levels
+// outside 1..max(trace_limit, 1), more than 2^28 path pixels (or visibility entries), and a light count other than the scene's
+static int checkPaths(cgrt_scene* s, const cgrt_camera* cams, int32_t nViews, const cgrt_render_params* p, int32_t nLevels,
+                      int32_t nLights, const float* rgb, const cgrt_path_buffers* paths)
+{
+    RC(checkViews(s, cams, nViews, p, rgb));
+    if (!paths) return fail(CGRT_ERR_INVALID, "null paths");
+    if (!paths->ray && !paths->depth && !paths->tri && !paths->normal && !paths->position && !paths->visibility)
+        return fail(CGRT_ERR_INVALID, "cgrt_render_paths: no buffer requested");
+    if (nLevels < 1 || nLevels > std::max(p->trace_limit, 1)) return fail(CGRT_ERR_INVALID, "n_levels must be in 1..max(trace_limit, 1)");
+    const int64_t px = (int64_t)nLevels * nViews * p->width * p->height;
+    if (px > (int64_t)1 << 28) return fail(CGRT_ERR_INVALID, "paths too large: n_levels x n_views x width x height > 2^28");
+    if (paths->visibility && px * nLights > (int64_t)1 << 28)
+        return fail(CGRT_ERR_INVALID, "visibility too large: n_levels x n_views x width x height x n_lights > 2^28");
+    size_t have;
+    {
+        std::lock_guard<std::mutex> lk(s->mu);
+        have = s->lights.size() + s->sphLights.size() / 7;
+    }
+    if (nLights < 0 || (size_t)nLights != have) return fail(CGRT_ERR_INVALID, "n_lights must be the scene's point plus spherical lights");
+    return CGRT_OK;
+}
+
+// the pass's buffers for cgrt_render_paths (device pointers)
+static AovBuffers pathAovs(const cgrt_path_buffers& d, int32_t nViews, const cgrt_render_params* p, int32_t nLevels, int32_t nLights)
+{
+    return AovBuffers{d.depth, d.tri, d.normal, nullptr, (float4*)d.ray, d.position, d.visibility, nLevels,
+                      (size_t)nViews * p->width * p->height, nLights};
+}
+
+int cgrt_render_paths_device(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, const cgrt_render_params* p,
+                             int32_t n_levels, int32_t n_lights, float* d_rgb, const cgrt_path_buffers* d_paths, void* stream)
+{
+    RC(checkPaths(s, cams, n_views, p, n_levels, n_lights, d_rgb, d_paths));
+    const AovBuffers A = pathAovs(*d_paths, n_views, p, n_levels, n_lights);
+    return renderDevice(s, cams, n_views, p, d_rgb, stream, &A);
 }
 
 // One frame's ray statistics (primary, primary_hit, shadow, bounce, replayed_*, pipeline) into a zeroed *stats: counts = its counters
@@ -1954,7 +1994,8 @@ int cgrt_render_aovs(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, co
         stage = s->aovStage.p;
     }
     const AovBuffers A = {aov->depth ? stage : nullptr, aov->tri ? (int*)(stage + px) : nullptr,
-                          aov->normal ? stage + 2 * px : nullptr, aov->hits ? (uint8_t*)(stage + 5 * px) : nullptr};
+                          aov->normal ? stage + 2 * px : nullptr, aov->hits ? (uint8_t*)(stage + 5 * px) : nullptr,
+                          nullptr, nullptr, nullptr, 1, 0, -1};
     RC(renderDevice(s, cams, n_views, p, s->frame.p, s->stream, &A));
     CK(cudaMemcpyAsync(rgb, s->frame.p, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, s->stream));
     if (aov->depth) CK(cudaMemcpyAsync(aov->depth, A.depth, px * sizeof(float), cudaMemcpyDeviceToHost, s->stream));
@@ -1986,6 +2027,47 @@ int cgrt_render_lights(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, 
     RC(renderDevice(s, cams, n_views, p, s->frame.p, s->stream, nullptr, &G));
     CK(cudaMemcpyAsync(rgb, s->frame.p, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, s->stream));
     CK(cudaMemcpyAsync(groups, stage, px * 3 * n_groups * sizeof(float), cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaStreamSynchronize(s->stream));
+    if (stats) RC(cgrt_render_collect_stats(s, stats));
+    return CGRT_OK;
+}
+
+// ---- every level of each pixel's mirror path ----------------------------------------------------------------------------------
+int cgrt_render_paths(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, const cgrt_render_params* p, int32_t n_levels,
+                      int32_t n_lights, float* rgb, const cgrt_path_buffers* paths, cgrt_render_stats* stats)
+{
+    RC(checkPaths(s, cams, n_views, p, n_levels, n_lights, rgb, paths));
+    RC(useSceneDevice(s));
+    std::lock_guard<std::mutex> hostLock(s->hostMu);
+    const size_t px = (size_t)n_views * p->width * p->height, n = px * n_levels;
+    // staging on the device, the requested buffers only, in this order (the rays first: 16-byte aligned)
+    struct Part {
+        void* host;
+        size_t floats;
+    } parts[6] = {{paths->ray, n * 8}, {paths->depth, n}, {paths->tri, n}, {paths->normal, n * 3}, {paths->position, n * 3},
+                  {paths->visibility, n * n_lights}};
+    size_t total = 0;
+    for (const Part& q : parts) total += q.host ? q.floats : 0;
+    float* stage = nullptr;
+    {
+        std::lock_guard<std::mutex> lk(s->mu);
+        RC(s->frame.ensure(px * 3));
+        RC(s->aovStage.ensure(total));
+        stage = s->aovStage.p;
+    }
+    void* dev[6];
+    size_t at = 0;
+    for (int k = 0; k < 6; k++) {
+        dev[k] = parts[k].host ? stage + at : nullptr;
+        at += parts[k].host ? parts[k].floats : 0;
+    }
+    const cgrt_path_buffers d = {(cgrt_ray*)dev[0], (float*)dev[1], (int32_t*)dev[2], (float*)dev[3], (float*)dev[4], (float*)dev[5]};
+    const AovBuffers A = pathAovs(d, n_views, p, n_levels, n_lights);
+    RC(renderDevice(s, cams, n_views, p, s->frame.p, s->stream, &A));
+    CK(cudaMemcpyAsync(rgb, s->frame.p, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, s->stream));
+    for (int k = 0; k < 6; k++)
+        if (parts[k].host && parts[k].floats)
+            CK(cudaMemcpyAsync(parts[k].host, dev[k], parts[k].floats * sizeof(float), cudaMemcpyDeviceToHost, s->stream));
     CK(cudaStreamSynchronize(s->stream));
     if (stats) RC(cgrt_render_collect_stats(s, stats));
     return CGRT_OK;

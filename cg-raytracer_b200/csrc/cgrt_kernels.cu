@@ -1896,53 +1896,103 @@ __global__ void k_generate_rays(const FrameParams* __restrict__ Pp, float4* __re
     rays[2 * (size_t)i + 1] = make_float4(d.x, d.y, d.z, 0.0f);
 }
 
-// ---- per-pixel buffers (cgrt_render_aovs) from the level-0 hit records ---------------------------------------------------------
-// The primary rays of a frame are those of k_generate_rays and its level-0 records hold what writeHit reports for them, so the
-// buffers equal cgrt_intersect_closest on cgrt_generate_rays bit for bit. r == nullptr: the primary ray missed.
-RT_DEV void storeAov(const DevScene& S, const AovBuffers& A, int outIdx, int depth, const float4* __restrict__ r)
+// ---- per-pixel buffers (cgrt_render_aovs) and mirror paths (cgrt_render_paths) from the hit records ----------------------------
+// The primary rays of a frame are those of k_generate_rays, each reflection ray is reflectionRayOf on the record before it (as
+// the frame's finish code builds it), and a record holds what writeHit reports for its ray, so every level equals
+// cgrt_intersect_closest on that level's ray bit for bit. A level without a ray (a miss or a non-mirror before it, the trace
+// limit) reports FLT_MAX, -1, 0 and a ray of +0.
+// rec: the index of the chain's first record (chain * levels); only its first `depth` records are read, the ones past them are
+// stale. cast, o, d, tIn: level 0's ray (cast = false: limit 0, no ray); ray0 = false: the caller wrote level 0's ray already.
+RT_DEV void storeAov(const DevScene& S, const FrameParams& P, const AovBuffers& A, int outIdx, int depth, const float4* __restrict__ hitRec,
+                     const uint8_t* __restrict__ lit, const float* __restrict__ soft, size_t rec, bool cast, V3 o, V3 d, float tIn,
+                     bool ray0)
 {
-    float t = FLT_MAX;
-    int id = -1;
-    float4 n = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
-    if (r) {
-        n = r[1];
-        t = n.w;
-        id = f2i(r[2].w);
-        if (id >= 0) id = f2i(__ldg(S.triV0 + id).w); // leaf order -> global id, as writeHit
-    }
-    if (A.depth) A.depth[outIdx] = t;
-    if (A.tri) A.tri[outIdx] = id;
-    if (A.normal) {
-        A.normal[3 * (size_t)outIdx] = n.x;
-        A.normal[3 * (size_t)outIdx + 1] = n.y;
-        A.normal[3 * (size_t)outIdx + 2] = n.z;
+    const int nL = P.nLights, nV = P.nLights + P.nSph;
+    for (int l = 0; l < A.levels; l++, rec++) {
+        const size_t i = (size_t)l * A.levelPixels + outIdx;
+        const bool hit = l < depth;
+        float t = cast ? tIn : FLT_MAX;
+        int id = -1;
+        float4 p = make_float4(0.0f, 0.0f, 0.0f, 0.0f), n = p, dr = p;
+        if (hit) {
+            const float4* r = hitRec + 3 * rec;
+            p = r[0];
+            n = r[1];
+            dr = r[2];
+            t = n.w;
+            id = f2i(dr.w);
+            if (id >= 0) id = f2i(__ldg(S.triV0 + id).w); // leaf order -> global id, as writeHit
+        }
+        if (A.ray && (l > 0 || ray0)) {
+            A.ray[2 * i] = cast ? make_float4(o.x, o.y, o.z, tIn) : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+            A.ray[2 * i + 1] = cast ? make_float4(d.x, d.y, d.z, 0.0f) : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+        }
+        if (A.depth) A.depth[i] = t;
+        if (A.tri) A.tri[i] = id;
+        if (A.normal) {
+            A.normal[3 * i] = n.x;
+            A.normal[3 * i + 1] = n.y;
+            A.normal[3 * i + 2] = n.z;
+        }
+        if (A.position) {
+            A.position[3 * i] = p.x;
+            A.position[3 * i + 1] = p.y;
+            A.position[3 * i + 2] = p.z;
+        }
+        if (A.visibility) { // the factors directColour applies: lit flag, then soft-shadow fraction
+            float* vis = A.visibility + i * nV;
+            for (int k = 0; k < nL; k++) vis[k] = hit && lit[rec * nL + k] ? 1.0f : 0.0f;
+            for (int k = 0; k < P.nSph; k++) vis[nL + k] = hit ? soft[rec * P.nSph + k] : 0.0f;
+        }
+        // the ray of level l + 1: shade()'s reflection ray off a mirror (main.cpp:246-256), below the trace limit (:267)
+        cast = false;
+        if (hit && l + 1 < A.levels) {
+            const int mat = f2i(p.w);
+            const float ksz = mat >= 0 ? __ldg(S.mats + 2 * mat + 1).z : 0.0f;
+            if (!(ksz <= 0.01f) && l + 1 < P.traceLimit) {
+                reflectionRayOf(mk3(p), mk3(dr), mk3(n), o, d, tIn);
+                cast = true;
+            }
+        }
     }
     if (A.hits) A.hits[outIdx] = (uint8_t)depth;
 }
 
-// one thread per pixel slot (padding slots of edge tiles write nothing); pathDepth == nullptr: every pixel is a miss
-__global__ void __launch_bounds__(128) k_aov_slots(DevScene S, const FrameParams* __restrict__ Pp, const float4* __restrict__ hitRec,
-                                                   const int* __restrict__ pathDepth, const int2* __restrict__ tileSeq, AovBuffers A)
+// one thread per pixel slot (padding slots of edge tiles write nothing); pathDepth == nullptr: every pixel is a miss. Level 0's
+// ray is the primary ray of the slot's view (k_gen / k_wave phase A)
+__global__ void __launch_bounds__(128) k_aov_slots(DevScene S, const FrameParams* __restrict__ Pp, const float4* __restrict__ lights,
+                                                   const float4* __restrict__ hitRec, const uint8_t* __restrict__ lit,
+                                                   const float* __restrict__ soft, const int* __restrict__ pathDepth,
+                                                   const int2* __restrict__ tileSeq, AovBuffers A)
 {
     const FrameParams P = *Pp;
     const int levels = P.traceLimit > 1 ? P.traceLimit : 1;
     for (int slot = blockIdx.x * blockDim.x + threadIdx.x; slot < P.nSlots; slot += gridDim.x * blockDim.x) {
-        int x, y, outIdx, local;
-        if (!seqToPixel(P, tileSeq, slot, x, y, outIdx, local)) continue;
-        const int depth = pathDepth ? pathDepth[slot] : 0;
-        storeAov(S, A, outIdx, depth, depth > 0 ? hitRec + 3 * (size_t)slot * levels : nullptr);
+        int x, y, outIdx, local, v;
+        if (!seqToPixel(P, tileSeq, slot, x, y, outIdx, local, v)) continue;
+        V3 o = mk3(0.0f, 0.0f, 0.0f), d = o;
+        if (A.ray && P.traceLimit > 0) {
+            const ViewCamera C = viewCamera(P, lights, v);
+            o = C.o;
+            d = primaryDirection(P, C, x, y);
+        }
+        storeAov(S, P, A, outIdx, pathDepth ? pathDepth[slot] : 0, hitRec, lit, soft, (size_t)slot * levels, P.traceLimit > 0, o, d,
+                 FLT_MAX, true);
     }
 }
 
-// path pipeline: one thread per path (primary rays that hit), after k_aov_slots has written every pixel as a miss
+// path pipeline: one thread per path (primary rays that hit), after k_aov_slots has written every pixel as a miss and its
+// level-0 ray
 __global__ void __launch_bounds__(128) k_aov_paths(DevScene S, const FrameParams* __restrict__ Pp, const float4* __restrict__ hitRec,
-                                                   const int* __restrict__ pathDepth, const int* __restrict__ pathPix,
-                                                   const int* __restrict__ counts, AovBuffers A)
+                                                   const uint8_t* __restrict__ lit, const int* __restrict__ pathDepth,
+                                                   const int* __restrict__ pathPix, const int* __restrict__ counts, AovBuffers A)
 {
-    const int levels = Pp->traceLimit > 1 ? Pp->traceLimit : 1;
+    const FrameParams P = *Pp;
+    const int levels = P.traceLimit > 1 ? P.traceLimit : 1;
     const int n = counts[CGRT_CNT_PATHS];
+    const V3 z = mk3(0.0f, 0.0f, 0.0f);
     for (int path = blockIdx.x * blockDim.x + threadIdx.x; path < n; path += gridDim.x * blockDim.x)
-        storeAov(S, A, pathPix[path], pathDepth[path], hitRec + 3 * (size_t)path * levels);
+        storeAov(S, P, A, pathPix[path], pathDepth[path], hitRec, lit, nullptr, (size_t)path * levels, true, z, z, FLT_MAX, false);
 }
 
 // ---- light groups (cgrt_render_lights) from the hit records, lit flags and soft-shadow fractions the frame left -----------------
@@ -2633,17 +2683,17 @@ int launchWavePipeline(const DevScene& S, const FrameParams* dP, const FramePara
     return 1;
 }
 
-int launchAovPass(const DevScene& S, const FrameParams* dP, const FrameParams& hP, const float4* hitRec, const int* pathDepth,
-                  bool perPath, const int* pathPix, const int* counts, const int2* dTileSeq, const AovBuffers& A, int numSMs,
-                  cudaStream_t st)
+int launchAovPass(const DevScene& S, const FrameParams* dP, const FrameParams& hP, const float4* dLights, const float4* hitRec,
+                  const uint8_t* lit, const float* soft, const int* pathDepth, bool perPath, const int* pathPix, const int* counts,
+                  const int2* dTileSeq, const AovBuffers& A, int numSMs, cudaStream_t st)
 {
     const int grid = gridFor((size_t)hP.nSlots, 128, numSMs * 16);
     if (!perPath || !pathDepth) {
-        k_aov_slots<<<grid, 128, 0, st>>>(S, dP, hitRec, pathDepth, dTileSeq, A);
+        k_aov_slots<<<grid, 128, 0, st>>>(S, dP, dLights, hitRec, lit, soft, pathDepth, dTileSeq, A);
         return 1;
     }
-    k_aov_slots<<<grid, 128, 0, st>>>(S, dP, hitRec, nullptr, dTileSeq, A); // the misses have no record
-    k_aov_paths<<<grid, 128, 0, st>>>(S, dP, hitRec, pathDepth, pathPix, counts, A);
+    k_aov_slots<<<grid, 128, 0, st>>>(S, dP, dLights, hitRec, lit, soft, nullptr, dTileSeq, A); // the misses have no record
+    k_aov_paths<<<grid, 128, 0, st>>>(S, dP, hitRec, lit, pathDepth, pathPix, counts, A);
     return 2;
 }
 

@@ -154,14 +154,23 @@ struct RoundBuffers {
     unsigned softSeed;
 };
 // hitRecordId: D.w of a hit record (bit-cast int) = the triangle's LEAF-ORDER index (global id: triV0[id].w), or -2 - s for
-// sphere s. N.w = t of the hit. The shading passes read neither lane; the AOV pass reads both from the level-0 records.
+// sphere s. N.w = t of the hit. The shading passes read neither lane; the AOV pass reads both.
 
-// Per-pixel buffers of a frame (cgrt_render_aovs), Screen layout, view after view; a null pointer is not written.
+// Per-pixel buffers of a frame (cgrt_render_aovs, cgrt_render_paths), Screen layout, view after view; a null pointer is not
+// written. Level l of the pixel's mirror path (the ray trace(l) cast and its hit) is at pixel l * levelPixels + the pixel's
+// index; cgrt_render_aovs is the one-level case without ray, position and visibility.
 struct AovBuffers {
-    float* depth;   // t of the primary ray's closest hit, FLT_MAX on a miss
-    int* tri;       // global triangle id of that hit, -1 miss, -2 - s sphere s
-    float* normal;  // 3 floats: shading normal of that hit, 0 on a miss
-    uint8_t* hits;  // levels of the pixel's path that recorded a hit (pathDepth)
+    float* depth;   // t of the level's closest hit; the ray's t on a miss, FLT_MAX where the level cast no ray
+    int* tri;       // global triangle id of that hit, -1 miss or no ray, -2 - s sphere s
+    float* normal;  // 3 floats: shading normal of that hit, 0 on a miss or no ray
+    uint8_t* hits;  // levels of the pixel's path that recorded a hit (pathDepth); one per pixel, not per level
+    float4* ray;        // 2 float4s: the level's ray [origin | t] [direction | 0]; all +0 where the level cast no ray
+    float* position;    // 3 floats: the hit record's P (the point shading() used), 0 where the level did not hit
+    float* visibility;  // nLights floats: each light's shadow factor at that point, point lights then spherical lights (1 / 0
+                        // lit / shadowed, k / 200 of the soft-shadow samples), 0 where the level did not hit
+    int levels;         // levels written (1..max(trace limit, 1))
+    size_t levelPixels; // pixels of all views
+    int nLights;        // cgrt_render_paths: the caller's light count, checked again when the frame reads the lights; -1: not given
 };
 
 // Light-group buffers of a frame (cgrt_render_lights): group g's [n_views][H][W][3] at rgb + g * groupFloats, Screen layout.
@@ -256,12 +265,13 @@ int waveGridBlocks(int numSMs); // co-resident CTAs of k_wave on this device (oc
 int launchWavePipeline(const DevScene& S, const FrameParams* dP, const FrameParams& hP, const float4* dLights,
                        const RoundBuffers& B, const WaveQ& Q, const int2* dTileSeq, float* fb, int numSMs, WaveTrace* tr,
                        cudaStream_t st);
-// The AOV pass after a frame of the path, round or wave pipeline (whole frames in Screen layout). pathDepth == nullptr: no
-// records (trace limit 0), every pixel is a miss; perPath: the path pipeline's records (per path, pathPix gives the pixel),
-// else one record chain per pixel slot. Returns the kernels it launched.
-int launchAovPass(const DevScene& S, const FrameParams* dP, const FrameParams& hP, const float4* hitRec, const int* pathDepth,
-                  bool perPath, const int* pathPix, const int* counts, const int2* dTileSeq, const AovBuffers& A, int numSMs,
-                  cudaStream_t st);
+// The AOV / mirror-path pass after a frame of the path, round or wave pipeline (whole frames in Screen layout). pathDepth ==
+// nullptr: no records (trace limit 0), every pixel is a miss; perPath: the path pipeline's records (per path, pathPix gives the
+// pixel), else one record chain per pixel slot. lit / soft: the frame's lit flags and soft-shadow fractions (read for
+// A.visibility only; soft: the round pipeline with spherical lights). Returns the kernels it launched.
+int launchAovPass(const DevScene& S, const FrameParams* dP, const FrameParams& hP, const float4* dLights, const float4* hitRec,
+                  const uint8_t* lit, const float* soft, const int* pathDepth, bool perPath, const int* pathPix, const int* counts,
+                  const int2* dTileSeq, const AovBuffers& A, int numSMs, cudaStream_t st);
 // The light-group pass after a frame of the path, round or wave pipeline with trace limit > 0 (whole frames in Screen layout).
 // perPath: the path pipeline's records, written through pathPix into buffers the caller has cleared to +0 (misses have no
 // record); else every pixel slot's chain, misses included. soft: the round pipeline's soft-shadow fractions (spherical lights).

@@ -285,6 +285,53 @@ int cgrt_render_aovs(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, co
                      const cgrt_aov_buffers* aov, cgrt_render_stats* stats);
 int cgrt_render_aovs_device(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, const cgrt_render_params* p,
                             float* d_rgb, const cgrt_aov_buffers* d_aov, void* stream);
+/* Mirror paths and shadow factors: every level of each pixel's getFinalColor recursion (the ray trace(level) cast, what it hit
+ * and where) and, at each hit, each light's shadow factor. Any pointer may be NULL: that buffer is not produced. */
+typedef struct cgrt_path_buffers {
+    cgrt_ray* ray;       /* [n_levels][n_views][H][W]           the ray trace(level) cast */
+    float* depth;        /* [n_levels][n_views][H][W]           t of its closest hit */
+    int32_t* tri;        /* [n_levels][n_views][H][W]           cgrt_hit.tri of that hit */
+    float* normal;       /* [n_levels][n_views][H][W][3]        cgrt_hit.normal of that hit */
+    float* position;     /* [n_levels][n_views][H][W][3]        the shading point of the hit */
+    float* visibility;   /* [n_levels][n_views][H][W][n_lights] each light's shadow factor at the hit */
+} cgrt_path_buffers;
+/* cgrt_render_views with the frame's mirror paths: the frame keeps one hit record per pixel and level, one lit flag per record
+ * and point light and (round pipeline) one soft-shadow fraction per record and spherical light; one pass after the frame walks
+ * each pixel's records and writes the requested buffers (DESIGN.md 4.5).
+ *   Layout   every buffer is in Screen layout (row H-1-y), view after view, level after level: level l of pixel (x, y) of view
+ *            v is element (l * n_views + v) * H * W + (H-1-y) * W + x. Lights come in the order of cgrt_render_lights: the
+ *            point lights (cgrt_scene_set_lights order), then the spherical lights.
+ *   Equality rgb is bit for bit what cgrt_render_views returns for the same arguments; so are the stats, except
+ *            kernel_launches, which also counts the pass (device_ms covers it).
+ *   Contract for level l of pixel (x, y) of view v:
+ *            (1) ray: level 0 is the ray of cgrt_generate_rays(cams[v]) whenever trace_limit > 0. Level l >= 1 exists when
+ *            level l-1 hit, that hit's material has ks.z > 0.01 and l < trace_limit: it is shade()'s reflection ray off the
+ *            level l-1 hit, origin P + 0.001 r, direction r = normalize(reflect(D, N)), t = |D| with D the incoming direction
+ *            (src/main.cpp:246-256). A level for which the recursion cast no ray (a miss or a non-mirror before it, the trace
+ *            limit, limit 0) is all +0 in ray.
+ *            (2) hit: depth, tri and normal are bit for bit what cgrt_intersect_closest returns for ray[l], so a miss reports
+ *            the ray's own t (FLT_MAX for a primary ray), tri -1 and normal 0. A level without a ray reports FLT_MAX, -1 and
+ *            0. Level 0 is therefore bit for bit the depth / tri / normal of cgrt_render_aovs, limit 0 included.
+ *            (3) position: the hit's shading point origin + t * direction (src/main.cpp:164); 0 where the level did not hit.
+ *            (4) visibility: the factor that level's shading() applied to each light's diffuse + specular term: 1 or 0 for a
+ *            point light (lit, or pointInShadow), k / 200 for a spherical light whose k of 200 samples arrived (the frame's
+ *            own samples, cgrt_scene_set_spherical_lights); 0 where the level did not hit.
+ *            (5) every level of every pixel is written on every call: levels past a pixel's path hold no data of an earlier
+ *            frame.
+ *   Refused  (CGRT_ERR_INVALID, before any CUDA call): everything cgrt_render_views refuses (so whole frames only, no
+ *            CGRT_RENDER_COUNT, no CGRT_RENDER_SCREEN_LAYOUT), a null paths or one whose six pointers are all NULL, n_levels
+ *            outside 1..max(trace_limit, 1), n_levels x n_views x W x H > 2^28, a requested visibility with n_levels x n_views
+ *            x W x H x n_lights > 2^28, and n_lights other than the scene's point plus spherical lights (checked again when the
+ *            frame reads the lights, which may change in between).
+ * The host form stages the buffers on the device, copies rgb and each requested buffer back on the scene's stream and
+ * synchronises once. The _device form takes device pointers and is asynchronous on `stream`; its statistics come from
+ * cgrt_render_collect_stats.
+ * Measured on one B200 (1000 W power limit), every buffer, n_levels = trace limit: the pass adds 0.22-0.28 ms to a 1080p view
+ * (C3, trace limit 5: 1.076 vs 1.293 ms for one view, 0.738 vs 1.018 ms per view for 8; DESIGN.md 4.5). */
+int cgrt_render_paths(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, const cgrt_render_params* p, int32_t n_levels,
+                      int32_t n_lights, float* rgb, const cgrt_path_buffers* paths, cgrt_render_stats* stats);
+int cgrt_render_paths_device(cgrt_scene* s, const cgrt_camera* cams, int32_t n_views, const cgrt_render_params* p,
+                             int32_t n_levels, int32_t n_lights, float* d_rgb, const cgrt_path_buffers* d_paths, void* stream);
 /* Light groups: cgrt_render_views with each group's share of every pixel in its own buffer, so that a light's colour can be
  * edited (relit) without tracing the frame again. One pass after the frame shades the hit records, lit flags and soft-shadow
  * fractions the frame left once per group, with the frame's arithmetic, restricted to the group's lights (DESIGN.md 4.5).
